@@ -2,6 +2,7 @@
 """Benchmark of the tri-plane render hot path (BASELINE.json metric: ray-samples/sec).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mode fp32|bf16] [--legs a,b,...]
+                    [--dump-outputs DIR]
 
 A "step" is one ImportanceRenderer.forward over one batch of synthetic input of the BASELINE config-2 shape: 8 images x
 128^2 rays x (48 coarse + 48 importance) samples, 3x32x256^2 planes per image, random-init OSGDecoder.  One process per
@@ -46,6 +47,7 @@ METRIC = 'ray-samples/sec'
 WORKLOAD = 'config2: batch 8 x 128^2 rays x (48+48) samples, 3x32x256^2 fp32 planes/image'
 ALL_LEGS = ('cpu_baseline', 'gpu_baseline', 'train_step', 'config3', 'config4', 'config5', 'strong', 'gather_check',
             'h2d_ceiling')
+DUMP_MAX_BYTES = 64 << 20
 
 OPTS = {'ray_start': 2.25, 'ray_end': 3.3, 'box_warp': 1, 'depth_resolution': DC, 'depth_resolution_importance': DF,
         'disparity_space_sampling': False, 'clamp_mode': 'softplus'}        # train.py:312-313,328-332
@@ -150,6 +152,24 @@ def make_decoder(torch, pkg, dev, seed):
     return pkg.OSGDecoder(32, {'decoder_lr_mul': 1, 'decoder_output_dim': 32}).to(dev).requires_grad_(False)
 
 
+def dump_outputs(out_dir, outputs):
+    """--dump-outputs: what the last timed step returned -- rgb [N,M,32], depth [N,M,1], weight sum [N,M,1] -- as
+    out_dir/<name>.npy in float32, so that two builds can be compared output for output.  Inputs and noise are seeded, so
+    the same arguments give the same inputs.  Beyond 64 MB in all (N > 1 gathers every rank's images) every array keeps the
+    same fixed, seeded sample of rays, flattened to [rays, channels]."""
+    arrays = {name: np.ascontiguousarray(t.detach().cpu().numpy(), dtype=np.float32)
+              for name, t in zip(('rgb', 'depth', 'weight_sum'), outputs)}
+    total = sum(a.nbytes for a in arrays.values())
+    budget = DUMP_MAX_BYTES - 4096                   # room for the .npy headers
+    if total > budget:
+        rays = arrays['depth'].shape[0] * arrays['depth'].shape[1]
+        keep = np.sort(np.random.default_rng(0).choice(rays, rays * budget // total, replace=False))
+        arrays = {name: np.ascontiguousarray(a.reshape(rays, -1)[keep]) for name, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def cpu_model():
     try:
         for line in open('/proc/cpuinfo'):
@@ -184,7 +204,8 @@ def reference_cpu_forward(torch, n_img, res, seed=100, threads=None):
 def run_reference(args):
     """`--impl reference`: the unmodified reference's CPU implementation of the path, all host threads, on this arm's
     config.  A step is one ImportanceRenderer.forward over the 8-image batch; if the host is so slow that K + W such steps
-    would take more than ~4 minutes, a step renders the first k of the 8 images instead (stated in `sample`)."""
+    would take more than ~4 minutes, a step renders the first k of the 8 images instead (stated in `sample`).  With
+    --dump-outputs a step always renders all 8, so that the dumped arrays do not depend on the host's speed."""
     if int(os.environ.get('RANK', '0')) != 0:
         return 0
     import torch
@@ -194,15 +215,17 @@ def run_reference(args):
     t1 = time.perf_counter() - t0                      # one image, cold: an upper bound of the per-image cost
     budget = 240.0
     k = N_IMG
-    while k > 1 and (args.steps + args.warmup) * k * t1 > budget:
+    while not args.dump_outputs and k > 1 and (args.steps + args.warmup) * k * t1 > budget:
         k //= 2
     for _ in range(args.warmup):
         fwd(k)
     times = []
     for _ in range(args.steps):
         t0 = time.perf_counter()
-        fwd(k)
+        last = fwd(k)
         times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     dt = float(np.mean(times))
     value = k * per_image / dt
     sample = (f'{k} of the {N_IMG} images per step x {RES}^2 rays x ({DC}+{DF}) samples, 3x32x256^2 planes: the unmodified '
@@ -769,7 +792,12 @@ def main():
     ap.add_argument('--gather', default='peer', choices=['peer', 'nccl'],
                     help='N > 1: peer = the render kernel stores into every GPU\'s gather buffers over NVLink; '
                          'nccl = render, then an in-place all-gather (A/B)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the rgb / depth / weight sum of the last timed step to DIR/<name>.npy (float32, at most '
+                         '64 MB in all: a fixed, seeded sample of rays beyond that)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         return run_reference(args)
     legs = set(ALL_LEGS) if args.legs == 'all' else set() if args.legs == 'none' else set(args.legs.split(','))
@@ -839,10 +867,13 @@ def main():
     t_wall0 = time.time()
     ev0.record()
     for _ in range(args.steps):
-        step(record=True)
+        last = step(record=True)
     ev1.record()
     cx.barrier()
     sampler_clk.window(t_wall0, time.time())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    del last
     ms = ev0.elapsed_time(ev1) / args.steps
     clocks = sampler_clk.stop() if rank == 0 else None
     kern_ms = float(np.mean([a.elapsed_time(b) for a, b in kernel_events]))
