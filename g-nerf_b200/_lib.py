@@ -71,6 +71,9 @@ _SIGNATURES = {
     'tpr_render_train': (ctypes.c_int, [_P, c_int64, c_int32, c_int32, _P, _P, _P, c_int64, _P, _P, _P, _P,
                                         ctypes.POINTER(TprOptions), _P, _P, _P, _P, _P, _P, _P, _P, ctypes.POINTER(c_int32), _P,
                                         c_size_t, _P]),
+    'tpr_run_model_backward_scratch_bytes': (c_size_t, [c_int64, c_int64]),
+    'tpr_run_model_backward': (ctypes.c_int, [_P, c_int64, c_int32, c_int32, _P, _P, c_int64, c_double, _P, _P, _P, c_int32,
+                                              _P, _P, _P, c_size_t, _P]),
     'tpr_unpack_decoder_grad': (ctypes.c_int, [_P, c_float, c_float, c_float, c_float, _P, _P, _P, _P, _P]),
     'tpr_march_backward': (ctypes.c_int, [_P, _P, c_int32, c_int32, _P, _P, _P, _P, _P, _P, c_int32, c_int64, _P, _P, _P]),
     'tpr_sample_planes': (ctypes.c_int, [_P, c_int64, c_int32, c_int32, _P, c_int64, c_double, _P, _P]),

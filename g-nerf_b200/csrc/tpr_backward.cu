@@ -277,8 +277,8 @@ struct DecArgs {
   const float* colours;                 // [T,32], or (col_chunked != 0) [rays, 8, S, 4]
   int col_chunked;
   const float* features;                // [T,32] summed plane features kept by the forward, or NULL: gather them again
-  const float* gsig; const float* omega;// [T]
-  const float* g_rgb;                   // [rays,32]
+  const float* gsig; const float* omega;// [T] (point queries: omega unused)
+  const float* g_rgb;                   // [rays,32]; point queries: [T,32] or NULL (sigma only)
   long long total, pts_per_img; int S;
   float box_scale;
   float* g_planes;                      // packed, zero-initialised
@@ -312,7 +312,9 @@ __device__ __forceinline__ void pair_sync(int id) { asm volatile("bar.sync %0, 6
 
 // FAST = false: 3xTF32 (fp32-grade gradients, the parity mode).  FAST = true (decoder_precision = 'bf16', the caller's
 // reduced-precision mode): operands rounded to TF32 (round to nearest), one HMMA per product.
-template <bool FAST>
+// POINT = true: point queries (ImportanceRenderer.run_model under autograd), as in decode_backward_tc_kernel: colours and g_rgb
+// rows per point, GY colour = g_rgb x 1.002 x s(1-s), no omega; g_rgb == NULL reads no colours (sigma only).
+template <bool FAST, bool POINT>
 __global__ void __launch_bounds__(kBT, 2) decode_backward_kernel(const DecArgs a) {
   extern __shared__ uint8_t smem_raw[];
   Smem& s = *reinterpret_cast<Smem*>(smem_raw + ((16u - ((uint32_t)__cvta_generic_to_shared(smem_raw) & 15u)) & 15u));
@@ -321,6 +323,7 @@ __global__ void __launch_bounds__(kBT, 2) decode_backward_kernel(const DecArgs a
   const int grp = lane >> 3, sub = lane & 7;       // gather: 8 lanes per sample
   const int mt = warp >> 1, hf = warp & 1;         // row block of 16 samples, column half
   const int row0 = mt * 16;
+  const bool want_col = !POINT || a.g_rgb != nullptr;
   // ---- stage the decoder, split once
   for (int i = tid; i < kC * kHid; i += kBT) {
     const int k = i >> 6, j = i & 63;
@@ -347,8 +350,8 @@ __global__ void __launch_bounds__(kBT, 2) decode_backward_kernel(const DecArgs a
   for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
     const long long gs0 = tile * kT;
     const long long n0 = gs0 / a.pts_per_img, rem0 = gs0 - n0 * a.pts_per_img;
-    const long long ray0 = gs0 / a.S;
-    const int rr0 = (int)(gs0 - ray0 * a.S);
+    const long long ray0 = POINT ? 0 : gs0 / a.S;
+    const int rr0 = POINT ? 0 : (int)(gs0 - ray0 * a.S);
     // ---- taps of this warp's 8 samples x 3 planes (VR/renderer.py:39-65)
     if (lane < 24) {
       const int sl = lane / 3, p = lane - sl * 3, sr = row0 + 8 * hf + sl;
@@ -377,7 +380,7 @@ __global__ void __launch_bounds__(kBT, 2) decode_backward_kernel(const DecArgs a
     for (int it = 0; it < 2; ++it) {
       const int sr = row0 + 8 * hf + it * 4 + grp;
       const long long gsf = gs0 + sr;
-      const bool kept = a.features != nullptr;
+      const bool kept = !POINT && a.features != nullptr;        // (point queries: always gathered again)
       const float4* img = reinterpret_cast<const float4*>(a.planes + (size_t)s.simg[sr] * img_stride) + sub;
       float4 v[12];
       float4 fk = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -391,14 +394,15 @@ __global__ void __launch_bounds__(kBT, 2) decode_backward_kernel(const DecArgs a
       const long long gs = gs0 + sr;
       float gy[4] = {0.f, 0.f, 0.f, 0.f};
       float gs_sig = 0.0f;
-      if (gs < a.total) {
-        const long long ray = ray0 + (unsigned)(rr0 + sr) / (unsigned)a.S;
-        const float4 col = a.col_chunked
+      if (gs < a.total) gs_sig = __ldg(a.gsig + gs);
+      if (gs < a.total && want_col) {
+        const long long ray = POINT ? gs : ray0 + (unsigned)(rr0 + sr) / (unsigned)a.S;      // the row of g_rgb
+        const float4 col = (!POINT && a.col_chunked)
             ? __ldg(reinterpret_cast<const float4*>(a.colours + ray * a.S * 32) + sub * a.S + (gs - ray * a.S))
             : __ldg(reinterpret_cast<const float4*>(a.colours + gs * 32) + sub);
         const float4 A = __ldg(reinterpret_cast<const float4*>(a.g_rgb + ray * 32) + sub);
-        const float om = __ldg(a.omega + gs) * (2.0f * 1.002f);       // rgb*2-1 (VR/ray_marcher.py:55), sigmoid*1.002 (training/triplane.py:134)
-        gs_sig = __ldg(a.gsig + gs);
+        // rgb*2-1 (VR/ray_marcher.py:55), sigmoid*1.002 (training/triplane.py:134)
+        const float om = POINT ? 1.002f : __ldg(a.omega + gs) * (2.0f * 1.002f);
         const float cc[4] = {col.x, col.y, col.z, col.w}, aa[4] = {A.x, A.y, A.z, A.w};
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
@@ -678,16 +682,18 @@ int launch_bwd_march(const float* dc, const float* df, int Dc, int Df, const flo
   return (int)cudaGetLastError();
 }
 
+// point != 0: point queries (see decode_backward_kernel)
 int launch_bwd_decode(const float* planes, int H, int W, const float* dec, const float* pts, const float* colours, int col_chunked,
                       const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total, long long pts_per_img, int S,
-                      float box_scale, float* g_planes, float* g_dec, int fast, int skip, int sms, cudaStream_t st) {
+                      int point, float box_scale, float* g_planes, float* g_dec, int fast, int skip, int sms, cudaStream_t st) {
   bwd::DecArgs a;
   a.planes = planes; a.H = H; a.W = W; a.dec = dec; a.pts = pts; a.colours = colours; a.col_chunked = col_chunked; a.features = features; a.gsig = gsig; a.omega = omega;
   a.g_rgb = g_rgb; a.total = total; a.pts_per_img = pts_per_img; a.S = S; a.box_scale = box_scale; a.g_planes = g_planes;
   a.g_dec = g_dec;
   { const char* e = getenv("TPR_BWD_DEBUG"); a.debug = skip | (e ? atoi(e) : 0); }
   const size_t smem = sizeof(bwd::Smem) + 16;
-  void (*kern)(const bwd::DecArgs) = fast ? bwd::decode_backward_kernel<true> : bwd::decode_backward_kernel<false>;
+  void (*kern)(const bwd::DecArgs) = point ? (fast ? bwd::decode_backward_kernel<true, true> : bwd::decode_backward_kernel<false, true>)
+                                           : (fast ? bwd::decode_backward_kernel<true, false> : bwd::decode_backward_kernel<false, false>);
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
   const long long n_tiles = (total + bwd::kT - 1) / bwd::kT;

@@ -27,6 +27,11 @@
 // range kernel) before they are split into fp16 halves, and the results are scaled back exactly: fp16 has 5 exponent bits
 // and gradients come at any scale (loss scaling).
 //
+// Point queries (ImportanceRenderer.run_model under autograd; kPoint = true): the same kernel with the input rows indexed by
+// point instead of by ray -- colours = the forward's rgb [T,32], g_rgb [T,32], GYc = g_rgb x 1.002 x s(1-s) (the render formula
+// with ray = point and omega = 1/2), gsig = the upstream gradient of sigma (density_noise is additive).  With g_rgb == NULL
+// (sigma-only queries) the LOAD warps read no colours and the GYc halves of the input tiles stay the zeros written at start.
+//
 // Roles (25 warps, one CTA per SM):  0-7 LOAD (features / colours / upstream gradient -> operand tiles)
 //                                     8-15 SCATTER (the sample's 12 taps from its position, red.global.add.v4.f32 of GF x tap
 //                                           weight; one texel = one 128-byte line = eight lanes)
@@ -82,8 +87,8 @@ struct Args {
   const float* colours;                 // [T,32], or (col_chunked != 0) [rays, 8, S, 4] as tpr_render_train keeps them
   int col_chunked;
   const float* features;                // [T,32] kept by the forward, or NULL: gather again
-  const float* gsig; const float* omega;// [T]
-  const float* g_rgb;                   // [rays,32]
+  const float* gsig; const float* omega;// [T] (point queries: omega unused)
+  const float* g_rgb;                   // [rays,32]; point queries: [T,32] or NULL (sigma only)
   long long total, pts_per_img; int S;
   float box_scale;
   float* g_planes;                      // packed, zero-initialised; NULL: no scatter
@@ -153,7 +158,7 @@ __global__ void scale_kernel(const float* __restrict__ g_rgb, long long n_rgb, c
   (void)dec;
 }
 __global__ void scale_finish_kernel(const unsigned* __restrict__ acc, const float* __restrict__ dec, float* __restrict__ scale) {
-  // bound of |GYc| = |g_rgb| * 2 * 1.002 * omega * s(1-s) <= 0.501 |g_rgb|; of |GH| = |GYc| . sum_c |W2c| + |gsig| |w2s|
+  // bound of |GYc| = |g_rgb| * 2 * 1.002 * omega * s(1-s) <= 0.501 |g_rgb| (point queries: 1.002 s(1-s) <= 0.2505); of |GH| = |GYc| . sum_c |W2c| + |gsig| |w2s|
   __shared__ float col[64];
   const int j = threadIdx.x;
   if (j < 64) {
@@ -186,7 +191,7 @@ __global__ void scale_finish_kernel(const unsigned* __restrict__ acc, const floa
 #define PROF(slot) do { if (kProf) { const long long t1_ = clock64(); prof_acc[slot] += t1_ - prof_t; prof_t = t1_; } } while (0)
 #define PROF_FLUSH(first, last, cond) do { if (kProf && blockIdx.x == 0 && lane == 0 && (cond)) { for (int k_ = first; k_ <= last; ++k_) a.prof[k_] = prof_acc[k_]; } } while (0)
 // ---- the kernel ------------------------------------------------------------------------------------------------------------
-template <bool kProf>
+template <bool kProf, bool kPoint>
 __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const Args a) {
   extern __shared__ uint8_t smem_raw[];
   Smem& s = *reinterpret_cast<Smem*>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
@@ -222,6 +227,13 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
     reinterpret_cast<__half*>(s.w2c)[j * 64 + (((((32 + c) >> 3) ^ (j & 7)) << 3) | (c & 7))] = lo;
   }
   if (tid < 64) { s.b1[tid] = __ldg(a.dec + kB1Off + tid); s.w2s[tid] = __ldg(a.dec + kW2tOff + tid * kOutPad); }
+  if (kPoint && a.g_rgb == nullptr) {                         // sigma-only: the GYc halves (chunks 4-7 of every row) stay zero
+    for (int i = tid; i < 2 * 2 * kM * 4; i += kThreads) {
+      const int row = (i >> 2) & (kM - 1), tile = i >> 9;      // tile: buffer b = tile >> 1, hi / lo = tile & 1
+      uint8_t* t = (tile & 1) ? s.in[tile >> 1].lo : s.in[tile >> 1].hi;
+      *reinterpret_cast<uint4*>(t + row * 128 + (((4 + (i & 3)) ^ (row & 7)) << 4)) = make_uint4(0u, 0u, 0u, 0u);
+    }
+  }
   fence_proxy_async_smem();
   tcgen05_fence_before();
   __syncthreads();
@@ -255,8 +267,10 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
       // tile-uniform index arithmetic once (64-bit divisions), 32-bit per sample: a tile straddles at most two images when an
       // image has >= 128 points (the launcher checks that), and (rr0 + sr) / S is a 32-bit division
       const long long n0 = gs0 / a.pts_per_img, rem0 = gs0 - n0 * a.pts_per_img;
-      const long long ray0 = gs0 / a.S;
-      const unsigned rr0 = (unsigned)(gs0 - ray0 * a.S);
+      long long ray0 = 0;
+      unsigned rr0 = 0;
+      if (!kPoint) { ray0 = gs0 / a.S; rr0 = (unsigned)(gs0 - ray0 * a.S); }
+      const bool want_col = !kPoint || a.g_rgb != nullptr;    // (warp-uniform)
       float4 f[2], colq[2], Aq[2];
 #pragma unroll 1
       for (int half = 0; half < 2; ++half) {
@@ -281,16 +295,19 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
       float omq = 0.f, gsq = 0.f;
       colq[0] = colq[1] = Aq[0] = Aq[1] = make_float4(0.f, 0.f, 0.f, 0.f);
       if (gsc < a.total) {
-        const long long ray = ray0 + (rr0 + (unsigned)src) / (unsigned)a.S;
+        const long long ray = kPoint ? gsc : ray0 + (rr0 + (unsigned)src) / (unsigned)a.S;     // the row of g_rgb
+        if (want_col) {
 #pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const int chunk = cq + 4 * j;
-          colq[j] = a.col_chunked
-              ? __ldg(reinterpret_cast<const float4*>(a.colours + ray * a.S * 32) + chunk * a.S + (gsc - ray * a.S))
-              : __ldg(reinterpret_cast<const float4*>(a.colours + gsc * 32) + chunk);
-          Aq[j] = __ldg(reinterpret_cast<const float4*>(a.g_rgb + ray * 32) + chunk);
+          for (int j = 0; j < 2; ++j) {
+            const int chunk = cq + 4 * j;
+            colq[j] = (!kPoint && a.col_chunked)
+                ? __ldg(reinterpret_cast<const float4*>(a.colours + ray * a.S * 32) + chunk * a.S + (gsc - ray * a.S))
+                : __ldg(reinterpret_cast<const float4*>(a.colours + gsc * 32) + chunk);
+            Aq[j] = __ldg(reinterpret_cast<const float4*>(a.g_rgb + ray * 32) + chunk);
+          }
         }
-        omq = __ldg(a.omega + gsc); gsq = __ldg(a.gsig + gsc);
+        if (!kPoint) omq = __ldg(a.omega + gsc);
+        gsq = __ldg(a.gsig + gsc);
       }
       PROF(0);
       if (half == 0) mbar_wait_parked(&s.in_free[b], ((uint32_t)(i >> 1) & 1u) ^ 1u);   // the weight-gradient MMAs of tile i - 2 have read the tiles
@@ -299,10 +316,10 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
       for (int it = 0; it < 2; ++it) st_hilo4(s.in[b].hi, s.in[b].lo, warp * 16 + (2 * half + it) * 4 + grp, 0, sub, f[it]);
       {
         // rgb*2-1 (VR/ray_marcher.py:55), sigmoid*1.002 (training/triplane.py:134); times the operand scale
-        const float om = omq * (2.0f * 1.002f) * sc;
+        const float om = kPoint ? 1.002f * sc : omq * (2.0f * 1.002f) * sc;
         const float gsg = gsq * sc;
 #pragma unroll
-        for (int j = 0; j < 2; ++j) {
+        for (int j = 0; j < 2 && want_col; ++j) {
           const float cc[4] = {colq[j].x, colq[j].y, colq[j].z, colq[j].w}, aa[4] = {Aq[j].x, Aq[j].y, Aq[j].z, Aq[j].w};
           float g4[4];
 #pragma unroll
@@ -594,16 +611,17 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
 
 // Launch; returns cudaError_t (0 = ok) or -1 when the device cannot run it (the caller keeps the mma.sync kernel).
 // scale_buf: 4 floats of device scratch ([0..1] the power-of-two scale and its inverse, [2..3] the range accumulators).
+// point != 0: point queries (rows of colours / g_rgb per point, no omega, S unused; g_rgb may be NULL).
 int launch_bwd_decode_tc(const float* planes, int H, int W, const float* dec, const float* pts, const float* colours, int col_chunked,
                          const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total,
-                         long long pts_per_img, int S, float box_scale, float* g_planes, float* g_dec, float* scale_buf,
+                         long long pts_per_img, int S, int point, float box_scale, float* g_planes, float* g_dec, float* scale_buf,
                          int sms, int smem_optin, cudaStream_t st) {
   using namespace bwdtc;
   const size_t smem = sizeof(Smem) + 1024;
   if ((int)smem > smem_optin) return -1;
   cudaError_t e = cudaMemsetAsync(scale_buf + 2, 0, 2 * sizeof(float), st);
   if (e != cudaSuccess) return (int)e;
-  const long long n_rgb = (total / S) * 32;
+  const long long n_rgb = point ? (g_rgb ? total * 32 : 0) : (total / S) * 32;
   scale_kernel<<<sms * 4, 256, 0, st>>>(g_rgb, n_rgb, gsig, total, dec, reinterpret_cast<unsigned*>(scale_buf + 2));
   scale_finish_kernel<<<1, 64, 0, st>>>(reinterpret_cast<const unsigned*>(scale_buf + 2), dec, scale_buf);
   Args a;
@@ -615,8 +633,9 @@ int launch_bwd_decode_tc(const float* planes, int H, int W, const float* dec, co
     if (d & 2) a.g_dec = nullptr;
     a.lookahead = (d & 8) ? 0 : 1; }
   static const bool profile = getenv("TPR_BWD_PROFILE") != nullptr;
-  e = profile ? cudaFuncSetAttribute(decode_backward_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-              : cudaFuncSetAttribute(decode_backward_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  void (*kern)(const Args) = profile ? (point ? decode_backward_tc_kernel<true, true> : decode_backward_tc_kernel<true, false>)
+                                     : (point ? decode_backward_tc_kernel<false, true> : decode_backward_tc_kernel<false, false>);
+  e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
   if (pts_per_img < kM) return -1;                 // (a tile may straddle at most two images)
   const long long n_tiles = (total + kM - 1) / kM;
@@ -629,14 +648,14 @@ int launch_bwd_decode_tc(const float* planes, int H, int W, const float* dec, co
     long long* prof = nullptr; long long host[17];
     cudaMalloc(&prof, sizeof(host)); cudaMemsetAsync(prof, 0, sizeof(host), st);
     a.prof = prof;
-    decode_backward_tc_kernel<true><<<(unsigned)grid, kThreads, smem, st>>>(a);
+    kern<<<(unsigned)grid, kThreads, smem, st>>>(a);
     cudaStreamSynchronize(st);
     cudaMemcpy(host, prof, sizeof(host), cudaMemcpyDeviceToHost); cudaFree(prof);
     const long long tiles0 = (n_tiles + grid - 1) / grid;
     for (int k = 0; k < 17; ++k) fprintf(stderr, "[bwd profile] %-32s %8.0f cycles / tile\n", names[k], (double)host[k] / (double)tiles0);
     return (int)cudaGetLastError();
   }
-  decode_backward_tc_kernel<false><<<(unsigned)grid, kThreads, smem, st>>>(a);
+  kern<<<(unsigned)grid, kThreads, smem, st>>>(a);
   return (int)cudaGetLastError();
 }
 

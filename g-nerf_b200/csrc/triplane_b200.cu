@@ -34,11 +34,11 @@ int launch_bwd_march(const float* dc, const float* df, int Dc, int Df, const flo
                      long long n_rays_total, float* gsig, float* omega, int sms, cudaStream_t st);
 int launch_bwd_decode(const float* planes, int H, int W, const float* dec, const float* pts, const float* colours, int col_chunked,
                       const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total, long long pts_per_img, int S,
-                      float box_scale, float* g_planes, float* g_dec, int fast, int skip, int sms, cudaStream_t st);
+                      int point, float box_scale, float* g_planes, float* g_dec, int fast, int skip, int sms, cudaStream_t st);
 // tpr_backward_tc.cu: the decoder backward on tcgen05 (returns -1 if it cannot run here)
 int launch_bwd_decode_tc(const float* planes, int H, int W, const float* dec, const float* pts, const float* colours, int col_chunked,
                          const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total,
-                         long long pts_per_img, int S, float box_scale, float* g_planes, float* g_dec, float* scale_buf,
+                         long long pts_per_img, int S, int point, float box_scale, float* g_planes, float* g_dec, float* scale_buf,
                          int sms, int smem_optin, cudaStream_t st);
 int launch_unpack_decoder_grad(const float* gd, float g_w1, float g_b1, float g_w2, float g_b2, float* w1, float* b1, float* w2,
                                float* b2, cudaStream_t st);
@@ -1325,15 +1325,71 @@ int tpr_render_backward(const float* planes_packed, int64_t n_img, int32_t heigh
   const char* impl = getenv("TPR_BWD_IMPL");
   if (!(impl && strcmp(impl, "hmma") == 0)) {
     rc = launch_bwd_decode_tc(planes_packed, height, width, decoder_packed, pts, col_in, col_chunked, sample_features, gsig, omega, g_rgb, (long long)T,
-                              (long long)n_rays * S, S, (float)(2.0 / opt->box_warp), g_planes_packed, g_decoder_packed, scale_buf,
+                              (long long)n_rays * S, S, 0, (float)(2.0 / opt->box_warp), g_planes_packed, g_decoder_packed, scale_buf,
                               di.sms, di.smem_optin, st);
     if (rc > 0) return cuda_fail((cudaError_t)rc, "decode_backward_tc_kernel");
     if (rc == 0) return 0;
   }
   float* g_dec_out = g_decoder_packed ? g_decoder_packed : reinterpret_cast<float*>(scratch);      // (never written when skipped)
   rc = launch_bwd_decode(planes_packed, height, width, decoder_packed, pts, col_in, col_chunked, sample_features, gsig, omega, g_rgb, (long long)T,
-                         (long long)n_rays * S, S, (float)(2.0 / opt->box_warp), g_planes_packed, g_dec_out,
+                         (long long)n_rays * S, S, 0, (float)(2.0 / opt->box_warp), g_planes_packed, g_dec_out,
                          opt->flags == TPR_MLP_BF16, (g_planes_packed ? 0 : 1) | (g_decoder_packed ? 0 : 2), di.sms, st);
+  if (rc != 0) return cuda_fail((cudaError_t)rc, "decode_backward_kernel");
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------
+// backward of tpr_run_model (ImportanceRenderer.run_model under autograd): the decoder backward kernels of tpr_render_backward
+// in their point-query mode -- no march, no sort; the features are gathered again
+// ---------------------------------------------------------------------------------------
+size_t tpr_run_model_backward_scratch_bytes(int64_t n_img, int64_t n_pts) {
+  if (n_img <= 0 || n_pts <= 0) return 0;
+  // a zero g_sigma row [T] (used when g_sigma is NULL), the operand scale of the tcgen05 decoder backward
+  return align256((size_t)n_img * (size_t)n_pts * 4) + 256;
+}
+
+int tpr_run_model_backward(const float* planes_packed, int64_t n_img, int32_t height, int32_t width, const float* decoder_packed,
+                           const float* xyz, int64_t n_pts, double box_warp, const float* rgb, const float* g_rgb,
+                           const float* g_sigma, int32_t flags, float* g_planes_packed, float* g_decoder_packed, void* scratch,
+                           size_t scratch_bytes, void* stream) {
+  if (g_rgb && !rgb) return fail(TPR_E_NULL, "tpr_run_model_backward: g_rgb needs the forward's rgb");
+  if (!g_rgb && !g_sigma) return fail(TPR_E_NULL, "tpr_run_model_backward: g_rgb and g_sigma are both NULL");
+  if (!planes_packed || !decoder_packed || !xyz || (!g_planes_packed && !g_decoder_packed) || !scratch)
+    return fail(TPR_E_NULL, "tpr_run_model_backward: NULL pointer");
+  if (n_img <= 0 || n_pts <= 0 || height <= 0 || width <= 0) return fail(TPR_E_SHAPE, "tpr_run_model_backward: bad shape");
+  if ((long long)3 * height * width * kC >= (1ll << 32)) return fail(TPR_E_SHAPE, "tpr_run_model_backward: planes too large");
+  if (!(box_warp > 0)) return fail(TPR_E_OPTION, "tpr_run_model_backward: box_warp must be > 0");
+  if (flags != TPR_MLP_FP32 && flags != TPR_MLP_BF16 && flags != TPR_MLP_FFMA)
+    return fail(TPR_E_OPTION, "tpr_run_model_backward: unknown decoder flag");
+  if (scratch_bytes < tpr_run_model_backward_scratch_bytes(n_img, n_pts))
+    return fail(TPR_E_SCRATCH, "tpr_run_model_backward: scratch too small");
+  DeviceInfo di = device_info();
+  if (!di.ok) return fail(TPR_E_DEVICE, "tpr_run_model_backward: no CUDA device");
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long T = (long long)n_img * n_pts;
+  float* zero_gsig = (float*)scratch;
+  float* scale_buf = (float*)((uint8_t*)scratch + align256((size_t)T * 4));
+  cudaError_t e = cudaSuccess;
+  if (!g_sigma) e = cudaMemsetAsync(zero_gsig, 0, (size_t)T * sizeof(float), st);
+  if (e == cudaSuccess && g_planes_packed) e = cudaMemsetAsync(g_planes_packed, 0, (size_t)n_img * 3 * height * width * kC * sizeof(float), st);
+  if (e == cudaSuccess && g_decoder_packed) e = cudaMemsetAsync(g_decoder_packed, 0, kDecFloats * sizeof(float), st);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync");
+  const float* gsig = g_sigma ? g_sigma : zero_gsig;
+  const float box_scale = (float)(2.0 / box_warp);      // python float (VR/renderer.py:61)
+  // tcgen05 first, the mma.sync kernel when it refuses (fewer than 128 points per image, too little shared memory) or with
+  // TPR_BWD_IMPL=hmma -- as in tpr_render_backward
+  const char* impl = getenv("TPR_BWD_IMPL");
+  int rc;
+  if (!(impl && strcmp(impl, "hmma") == 0)) {
+    rc = launch_bwd_decode_tc(planes_packed, height, width, decoder_packed, xyz, rgb, 0, nullptr, gsig, nullptr, g_rgb, T, n_pts, 1, 1,
+                              box_scale, g_planes_packed, g_decoder_packed, scale_buf, di.sms, di.smem_optin, st);
+    if (rc > 0) return cuda_fail((cudaError_t)rc, "decode_backward_tc_kernel");
+    if (rc == 0) return 0;
+  }
+  float* g_dec_out = g_decoder_packed ? g_decoder_packed : reinterpret_cast<float*>(scratch);      // (never written when skipped)
+  rc = launch_bwd_decode(planes_packed, height, width, decoder_packed, xyz, rgb, 0, nullptr, gsig, nullptr, g_rgb, T, n_pts, 1, 1,
+                         box_scale, g_planes_packed, g_dec_out, flags == TPR_MLP_BF16, (g_planes_packed ? 0 : 1) | (g_decoder_packed ? 0 : 2),
+                         di.sms, st);
   if (rc != 0) return cuda_fail((cudaError_t)rc, "decode_backward_kernel");
   return 0;
 }

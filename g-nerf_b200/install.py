@@ -50,7 +50,8 @@ def install(reference_package: str = 'training.volumetric_rendering'):
     for attr, val in (('last_depth_range', None), ('last_fine', None), ('debug_outputs', False),
                       ('defer_depth_clamp', False), ('_timing_events', None), ('cache_packed_planes', False),
                       ('_plane_cache', None), ('_packed', _r.ImportanceRenderer._packed),
-                      ('_forward_impl', _r.ImportanceRenderer._forward_impl)):
+                      ('_forward_impl', _r.ImportanceRenderer._forward_impl),
+                      ('_run_model_impl', _r.ImportanceRenderer._run_model_impl)):
         setattr(ref_r.ImportanceRenderer, attr, val)
 
 

@@ -346,8 +346,14 @@ def run_model_sharded(renderer, planes, decoder, sample_coordinates, sample_dire
     [N,P,3]: rank r queries the r-th contiguous slab of the P points and sigma (4 bytes per point; plus rgb, 128 bytes,
     only when asked for) is all-gathered in place, so every rank returns the complete {'rgb', 'sigma'} of the reference.
     ``gather=False`` returns this rank's slab only (a caller that writes its own z-slab of an .mrc volume).
-    No collective touches the planes or the coordinates; density_noise is drawn per slab (each rank from its own generator)."""
-    world = dist.get_world_size(group) if dist.is_initialized() else 1
+    No collective touches the planes or the coordinates; density_noise is drawn per slab (each rank from its own generator).
+    Inference only: the in-place all-gather would drop the other ranks' share of any gradient, so autograd raises."""
+    if torch.is_grad_enabled():
+        tensors = [planes, sample_coordinates] + (list(decoder.parameters()) if isinstance(decoder, torch.nn.Module) else [])
+        if any(isinstance(t, torch.Tensor) and t.requires_grad for t in tensors):
+            raise NotImplementedError('run_model_sharded is inference-only (its all-gather carries no gradient): call it under '
+                                      'torch.no_grad() or use ImportanceRenderer.run_model for a differentiable query')
+    world =dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     n, p, _ = sample_coordinates.shape
     slabs = point_slabs(p, world)

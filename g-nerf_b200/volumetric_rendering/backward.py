@@ -1,4 +1,4 @@
-"""Autograd for ImportanceRenderer.forward: gradients w.r.t. the tri-planes and the OSGDecoder's four tensors.
+"""Autograd for ImportanceRenderer.forward and run_model: gradients w.r.t. the tri-planes and the OSGDecoder's four tensors.
 
 The reference gets its backward from PyTorch autograd over ~40 ATen ops and ~10 GB of saved activations per forward at
 FFHQ training shape (SURVEY.md section 3.2); training back-propagates through the renderer at
@@ -68,23 +68,30 @@ class _Render(torch.autograd.Function):
                                              p(s_feat) if ctx.has_feat else None,
                                              p(g_planes), p(g_dec), p(scratch), nbytes, st()),
                        'tpr_render_backward')
-            g_w1 = g_b1 = g_w2 = g_b2 = None
-            if want_dec:
-                g_w1 = torch.empty((64, 32), device=dev, dtype=torch.float32)
-                g_b1 = torch.empty(64, device=dev, dtype=torch.float32)
-                g_w2 = torch.empty((33, 64), device=dev, dtype=torch.float32)
-                g_b2 = torch.empty(33, device=dev, dtype=torch.float32)
-                _lib.check(L.tpr_unpack_decoder_grad(p(g_dec), *ctx.gains, p(g_w1), p(g_b1), p(g_w2), p(g_b2), st()),
-                           'tpr_unpack_decoder_grad')
-            g_nchw = None
-            if want_planes:
-                # the plane gradient was scattered in the packed layout [N,3,H,W,32]; the backbone wants [N,3,32,H,W] contiguous
-                # (autograd would otherwise make that copy itself, strided: 0.22 ms vs 0.08 ms for 201 MB at config 2)
-                g_nchw = torch.empty((n, 3, 32, pp.height, pp.width), device=dev, dtype=torch.float32)
-                _lib.check(L.tpr_unpack_planes(p(g_planes), n, pp.height, pp.width, p(g_nchw), st()), 'tpr_unpack_planes')
+            g_nchw, g_w1, g_b1, g_w2, g_b2 = _unpack_grads(g_planes, g_dec, ctx.gains, pp, dev)
         return (None, None, None, None, g_nchw,
                 g_w1 if need[5] else None, g_b1 if need[6] else None, g_w2 if need[7] else None, g_b2 if need[8] else None,
                 None, None)
+
+
+def _unpack_grads(g_planes, g_dec, gains, pp, dev):
+    """Packed gradients (either may be None) -> (planes [N,3,32,H,W], w1, b1, w2, b2) of the module's raw tensors."""
+    L, p, st = _lib.lib(), _r._ptr, _r._stream
+    g_w1 = g_b1 = g_w2 = g_b2 = None
+    if g_dec is not None:
+        g_w1 = torch.empty((64, 32), device=dev, dtype=torch.float32)
+        g_b1 = torch.empty(64, device=dev, dtype=torch.float32)
+        g_w2 = torch.empty((33, 64), device=dev, dtype=torch.float32)
+        g_b2 = torch.empty(33, device=dev, dtype=torch.float32)
+        _lib.check(L.tpr_unpack_decoder_grad(p(g_dec), *gains, p(g_w1), p(g_b1), p(g_w2), p(g_b2), st()),
+                   'tpr_unpack_decoder_grad')
+    g_nchw = None
+    if g_planes is not None:
+        # the plane gradient was scattered in the packed layout [N,3,H,W,32]; the backbone wants [N,3,32,H,W] contiguous
+        # (autograd would otherwise make that copy itself, strided: 0.22 ms vs 0.08 ms for 201 MB at config 2)
+        g_nchw = torch.empty((pp.n_img, 3, 32, pp.height, pp.width), device=dev, dtype=torch.float32)
+        _lib.check(L.tpr_unpack_planes(p(g_planes), pp.n_img, pp.height, pp.width, p(g_nchw), st()), 'tpr_unpack_planes')
+    return g_nchw, g_w1, g_b1, g_w2, g_b2
 
 
 def render_with_grad(renderer, planes, decoder, ray_origins, ray_directions, options, noise=None):
@@ -103,3 +110,66 @@ def render_with_grad(renderer, planes, decoder, ray_origins, ray_directions, opt
     fc1, fc2 = decoder.net[0], decoder.net[2]
     return _Render.apply(renderer, decoder, options, noise, planes, fc1.weight, fc1.bias, fc2.weight, fc2.bias,
                          ray_origins, ray_directions)
+
+
+class _RunModel(torch.autograd.Function):
+    """ImportanceRenderer.run_model with autograd: the forward is the inference point query (same kernel, same outputs, the
+    same density_noise draw); the backward is ``tpr_run_model_backward`` (the decoder backward kernels in their point-query
+    mode: no march, no sort, the features gathered again).  Saved: the packed planes and decoder, the coordinates and rgb."""
+
+    @staticmethod
+    def forward(ctx, renderer, decoder, options, want_rgb, sigma_noise, xyz, planes, w1, b1, w2, b2):
+        ctx.set_materialize_grads(False)           # an unused output hands in None: rgb unused = the sigma-only backward
+        with torch.no_grad():
+            out, aux = renderer._run_model_impl(planes.detach(), decoder, xyz, options, want_rgb=want_rgb,
+                                                sigma_noise=sigma_noise, train=True)
+        fc1, fc2 = decoder.net[0], decoder.net[2]
+        ctx.gains = (float(fc1.weight_gain), float(fc1.bias_gain), float(fc2.weight_gain), float(fc2.bias_gain))
+        ctx.packed, ctx.want_rgb = aux['packed'], want_rgb
+        ctx.box_warp, ctx.flags = float(options['box_warp']), _r._mlp_flag(options)
+        rgb, sigma = out['rgb'], out['sigma']
+        ctx.save_for_backward(aux['packed'].data, aux['dec'], aux['xyz'],
+                              rgb if want_rgb else torch.empty(0, device=sigma.device))
+        return (rgb, sigma) if want_rgb else sigma
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable          # raw CUDA kernels: a double backward must raise, not detach silently
+    def backward(ctx, *grads):
+        g_rgb, g_sigma = grads if ctx.want_rgb else (None, grads[0])
+        need = ctx.needs_input_grad
+        want_planes, want_dec = need[6], any(need[7:11])
+        if (g_rgb is None and g_sigma is None) or not (want_planes or want_dec):
+            return (None,) * 11
+        packed, dec, xyz, rgb = ctx.saved_tensors
+        pp, dev = ctx.packed, packed.device
+        n, npts, _ = xyz.shape
+        L, p, st = _lib.lib(), _r._ptr, _r._stream
+        g_rgb = g_rgb.contiguous().float() if g_rgb is not None else None
+        g_sigma = g_sigma.contiguous().float() if g_sigma is not None else None
+        with torch.cuda.device(dev):
+            g_planes = torch.empty_like(packed) if want_planes else None
+            g_dec = torch.empty_like(dec) if want_dec else None
+            nbytes = L.tpr_run_model_backward_scratch_bytes(n, npts)
+            scratch = torch.empty(nbytes, device=dev, dtype=torch.uint8)
+            _lib.check(L.tpr_run_model_backward(p(packed), n, pp.height, pp.width, p(dec), p(xyz), npts, ctx.box_warp,
+                                                p(rgb) if g_rgb is not None else None, p(g_rgb), p(g_sigma), ctx.flags,
+                                                p(g_planes), p(g_dec), p(scratch), nbytes, st()),
+                       'tpr_run_model_backward')
+            g_nchw, g_w1, g_b1, g_w2, g_b2 = _unpack_grads(g_planes, g_dec, ctx.gains, pp, dev)
+        return (None, None, None, None, None, None, g_nchw,
+                g_w1 if need[7] else None, g_b1 if need[8] else None, g_w2 if need[9] else None, g_b2 if need[10] else None)
+
+
+def run_model_with_grad(renderer, planes, decoder, sample_coordinates, options, want_rgb=True, sigma_noise=None):
+    """ImportanceRenderer.run_model with autograd: returns {'rgb', 'sigma'} attached to ``planes`` and to the decoder's
+    parameters (TriPlaneGenerator.sample / sample_mixed under a training step, e.g. EG3D's density regulariser)."""
+    if isinstance(planes, _r.PackedPlanes):
+        raise NotImplementedError('autograd needs the planes tensor itself ([N,3,32,H,W]), not PackedPlanes')
+    if isinstance(sample_coordinates, torch.Tensor) and sample_coordinates.requires_grad:
+        raise NotImplementedError('sample_coordinates requires grad: the renderer differentiates w.r.t. planes and decoder only')
+    _r.pack_decoder(decoder, allow_grad=True)            # validates the decoder's structure before anything is launched
+    fc1, fc2 = decoder.net[0], decoder.net[2]
+    out = _RunModel.apply(renderer, decoder, options, bool(want_rgb), sigma_noise, sample_coordinates, planes, fc1.weight,
+                          fc1.bias, fc2.weight, fc2.bias)
+    rgb, sigma = out if want_rgb else (None, out)
+    return {'rgb': rgb, 'sigma': sigma}

@@ -481,15 +481,25 @@ class ImportanceRenderer(torch.nn.Module):
     def run_model(self, planes, decoder, sample_coordinates, sample_directions, options, *, want_rgb=True, sigma_noise=None):
         """``sample_directions`` is accepted and ignored, exactly like OSGDecoder ignores it
         (training/triplane.py:124-136).  ``options['density_noise'] > 0`` adds ``randn_like(sigma) * density_noise``
-        (VR/renderer.py:146); ``sigma_noise`` [N,P,1] overrides the draw (tests)."""
+        (VR/renderer.py:146); ``sigma_noise`` [N,P,1] overrides the draw (tests).
+        Under autograd (planes or decoder parameters that require grad) the result is attached to them: this is the body of
+        TriPlaneGenerator.sample / sample_mixed (training/triplane.py:92-104), e.g. EG3D's density regulariser."""
+        if torch.is_grad_enabled() and _wants_grad(planes, decoder):
+            from .backward import run_model_with_grad
+            return run_model_with_grad(self, planes, decoder, sample_coordinates, options, want_rgb, sigma_noise)
+        return self._run_model_impl(planes, decoder, sample_coordinates, options, want_rgb=want_rgb, sigma_noise=sigma_noise)[0]
+
+    def _run_model_impl(self, planes, decoder, sample_coordinates, options, *, want_rgb=True, sigma_noise=None, train=False):
+        """The point query proper.  Returns ({'rgb', 'sigma'}, aux); ``train=True`` (the autograd path) lets the decoder
+        require grad and returns in ``aux`` what the backward needs: the packed planes and decoder and the coordinates."""
         xyz = _require_cuda_f32(sample_coordinates, 'sample_coordinates', (3,))
-        _forbid_autograd(planes if isinstance(planes, torch.Tensor) else None, xyz)
+        _forbid_autograd(None if train or not isinstance(planes, torch.Tensor) else planes, xyz)
         dn = _density_noise(options)
         pp = self._packed(planes)
         n, p, _ = xyz.shape
         if pp.n_img != n:
             raise RuntimeError(f'batch mismatch: planes N={pp.n_img}, coordinates N={n}')
-        dec = pack_decoder(decoder)
+        dec = pack_decoder(decoder, allow_grad=train)
         dev = xyz.device
         with torch.cuda.device(dev):
             rgb = torch.empty((n, p, 32), device=dev, dtype=torch.float32) if want_rgb else None
@@ -501,7 +511,8 @@ class ImportanceRenderer(torch.nn.Module):
                 nz = (torch.randn((n, p, 1), device=dev, dtype=torch.float32) if sigma_noise is None
                       else _require_cuda_f32(sigma_noise, 'sigma_noise').reshape(n, p, 1))
                 _lib.check(_lib.lib().tpr_add_density_noise(_ptr(sigma), _ptr(nz), n * p, dn, _stream()), 'tpr_add_density_noise')
-        return {'rgb': rgb, 'sigma': sigma}
+        aux = dict(packed=pp, dec=dec, xyz=xyz) if train else None
+        return {'rgb': rgb, 'sigma': sigma}, aux
 
     # ------------------------------------------------------------------ sort_samples / unify_samples (VR/renderer.py:150-167)
     def sort_samples(self, all_depths, all_colors, all_densities):

@@ -324,6 +324,23 @@ int tpr_render_train(const float* planes_packed, int64_t n_img, int32_t height, 
  * (the chain rule through the runtime gains, training/networks_stylegan2.py:118-127, and the plane mean's 1/3). */
 int tpr_unpack_decoder_grad(const float* g_decoder_packed, float w1_gain, float b1_gain, float w2_gain, float b2_gain,
                             float* g_w1, float* g_b1, float* g_w2, float* g_b2, void* stream);
+/* ---- backward of a8: ImportanceRenderer.run_model under autograd (TriPlaneGenerator.sample / sample_mixed,
+ *      training/triplane.py:92-104; e.g. EG3D's density regulariser) -------------------------------------------- */
+/* Gradients of L with respect to the tri-planes and the decoder, given g_rgb = dL/d(rgb) [N,P,32] and g_sigma = dL/d(sigma)
+ * [N,P] of one tpr_run_model call on the same planes, decoder, xyz, box_warp and flags.  rgb [N,P,32] is that call's rgb output
+ * (required with g_rgb).  Either upstream gradient may be NULL (= zero; not both): g_rgb = NULL is the sigma-only query and
+ * reads no colours.  density_noise is additive, so g_sigma is the gradient of the noise-free sigma too.  The features are
+ * gathered again (nothing per point is kept by the forward).  Either output may be NULL (not both); g_planes_packed
+ * [N,3,H,W,32] and g_decoder_packed are OVERWRITTEN, in the layouts of tpr_render_backward (convert with tpr_unpack_planes /
+ * tpr_unpack_decoder_grad).  flags: the forward's TPR_MLP_* (TPR_MLP_BF16 selects reduced-precision products where the
+ * mma.sync fall-back runs).  scratch: tpr_run_model_backward_scratch_bytes(n_img, n_pts) bytes. */
+size_t tpr_run_model_backward_scratch_bytes(int64_t n_img, int64_t n_pts);
+int tpr_run_model_backward(const float* planes_packed, int64_t n_img, int32_t height, int32_t width,
+                           const float* decoder_packed, const float* xyz /*[N,P,3]*/, int64_t n_pts, double box_warp,
+                           const float* rgb /*[N,P,32] or NULL*/, const float* g_rgb /*[N,P,32] or NULL*/,
+                           const float* g_sigma /*[N,P] or NULL*/, int32_t flags,
+                           float* g_planes_packed /*or NULL*/, float* g_decoder_packed /*or NULL*/,
+                           void* scratch, size_t scratch_bytes, void* stream);
 /* the two stages of tpr_render_backward, stand-alone (tests): the march's backward -- sigma [R,S], colours [R,S,32] of
  * the samples in forward order -> g_sigma [R,S] and the composite weight omega [R,S] of each sample's colour
  * (dL/d(colour_c) = 2 * g_rgb_c * omega) */
