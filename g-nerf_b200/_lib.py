@@ -13,6 +13,7 @@ from .build import LIB_PATH, BENCH_LIB_PATH
 
 ABI_VERSION = 8
 MLP_FP32, MLP_BF16, MLP_FFMA = 0, 1, 2
+BWD_DETERMINISTIC = 0x100          # OR-ed into the flags of the two backward entry points (TPR_BWD_DETERMINISTIC)
 LAYOUT_CHANNELS_LAST, LAYOUT_CHANNELS_FIRST = 0, 1
 
 
@@ -74,6 +75,7 @@ _SIGNATURES = {
     'tpr_run_model_backward_scratch_bytes': (c_size_t, [c_int64, c_int64]),
     'tpr_run_model_backward': (ctypes.c_int, [_P, c_int64, c_int32, c_int32, _P, _P, c_int64, c_double, _P, _P, _P, c_int32,
                                               _P, _P, _P, c_size_t, _P]),
+    'tpr_backward_deterministic_scratch_bytes': (c_size_t, [c_int64, c_int32, c_int32]),
     'tpr_unpack_decoder_grad': (ctypes.c_int, [_P, c_float, c_float, c_float, c_float, _P, _P, _P, _P, _P]),
     'tpr_march_backward': (ctypes.c_int, [_P, _P, c_int32, c_int32, _P, _P, _P, _P, _P, _P, c_int32, c_int64, _P, _P, _P]),
     'tpr_sample_planes': (ctypes.c_int, [_P, c_int64, c_int32, c_int32, _P, c_int64, c_double, _P, _P]),

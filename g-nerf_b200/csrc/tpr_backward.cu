@@ -286,6 +286,11 @@ struct DecArgs {
   int debug;                            // bit 0: no plane-gradient scatter, bit 1: no weight-gradient phase (the caller does not want
                                         // that gradient; TPR_BWD_DEBUG ORs into it for profiling A/B runs)
 };
+// DET (deterministic mode): the plane gradient goes to g_acc in fixed point (scale 2^e from det_hdr), the decoder gradient to
+// this CTA's row of dec_rows (a separate type, so that the default kernels' parameter block stays as it is)
+struct DetDecArgs : DecArgs {
+  unsigned long long* g_acc; float* dec_rows; int* det_hdr;
+};
 
 __device__ __forceinline__ void split_tf32(float x, uint32_t& hi, uint32_t& lo) {
   hi = __float_as_uint(x) & 0xffffe000u;          // the tensor core reads the top 19 bits of an fp32 register
@@ -314,8 +319,9 @@ __device__ __forceinline__ void pair_sync(int id) { asm volatile("bar.sync %0, 6
 // reduced-precision mode): operands rounded to TF32 (round to nearest), one HMMA per product.
 // POINT = true: point queries (ImportanceRenderer.run_model under autograd), as in decode_backward_tc_kernel: colours and g_rgb
 // rows per point, GY colour = g_rgb x 1.002 x s(1-s), no omega; g_rgb == NULL reads no colours (sigma only).
-template <bool FAST, bool POINT>
-__global__ void __launch_bounds__(kBT, 2) decode_backward_kernel(const DecArgs a) {
+// DET = true: the deterministic mode (DecArgs::g_acc).
+template <bool FAST, bool POINT, bool DET = false, class Args = DecArgs>
+__global__ void __launch_bounds__(kBT, 2) decode_backward_kernel(const Args a) {
   extern __shared__ uint8_t smem_raw[];
   Smem& s = *reinterpret_cast<Smem*>(smem_raw + ((16u - ((uint32_t)__cvta_generic_to_shared(smem_raw) & 15u)) & 15u));
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -561,6 +567,24 @@ __global__ void __launch_bounds__(kBT, 2) decode_backward_kernel(const DecArgs a
 #pragma unroll 1
     for (int it = 0; it < 2; ++it) {
       const int sr = row0 + 8 * hf + it * 4 + grp;
+      if constexpr (DET) {
+        // deterministic: GF x 2^e, four fixed-point reductions per lane and texel
+        if (a.debug & 1) continue;
+        const float fx = __int_as_float(__ldg(a.det_hdr + 2));
+        float4 gf = *reinterpret_cast<const float4*>(s.GF + sr * FS + 4 * sub);
+        gf = make_float4(gf.x * fx, gf.y * fx, gf.z * fx, gf.w * fx);
+        if (!fixed_ok(gf)) a.det_hdr[1] = 1;
+        unsigned long long* img = a.g_acc + (size_t)s.simg[sr] * img_stride + 4 * sub;
+#pragma unroll
+        for (int k = 0; k < 12; ++k) {
+          const float w = s.tap_w[sr * 12 + k];
+          if (w != 0.0f) {
+            unsigned long long* t = img + s.tap_off[sr * 12 + k];
+            red_add_fixed(t, w * gf.x); red_add_fixed(t + 1, w * gf.y); red_add_fixed(t + 2, w * gf.z); red_add_fixed(t + 3, w * gf.w);
+          }
+        }
+        continue;
+      }
       const float4 gf = *reinterpret_cast<const float4*>(s.GF + sr * FS + 4 * sub);
       float4* img = reinterpret_cast<float4*>(a.g_planes + (size_t)s.simg[sr] * img_stride) + sub;
 #pragma unroll
@@ -617,6 +641,27 @@ __global__ void __launch_bounds__(kBT, 2) decode_backward_kernel(const DecArgs a
 
   // ---- flush this CTA's partial weight gradients
   if (a.debug & 2) return;
+  if constexpr (DET) {
+    // deterministic: every element has one owning thread, which stores it into the CTA's row
+    float* drow = a.dec_rows + (size_t)blockIdx.x * kDecFloats;
+    const bool second = warp < 4;
+    const int pm = second ? warp : (warp - 4) >> 1;
+    const int pn0 = second ? 0 : 4 * ((warp - 4) & 1);
+#pragma unroll
+    for (int i = 0; i < 5; ++i) {
+      if (i < 4 || second) {
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+          const int m = 16 * pm + g + (r >> 1) * 8, n = 8 * (pn0 + i) + 2 * t + (r & 1);
+          if (!second) drow[kW1tOff + m * kHid + n] = pacc[i][r];
+          else if (n < kOutPad) drow[kW2tOff + m * kOutPad + n] = pacc[i][r];
+        }
+      }
+    }
+    if (tid < kHid) drow[kB1Off + tid] = bacc;
+    else if (tid < kHid + kOutPad) drow[kB2Off + tid - kHid] = bacc;
+    return;
+  }
   {
     const bool second = warp < 4;
     const int pm = second ? warp : (warp - 4) >> 1;
@@ -635,6 +680,27 @@ __global__ void __launch_bounds__(kBT, 2) decode_backward_kernel(const DecArgs a
   }
   if (tid < kHid) atomicAdd(a.g_dec + kB1Off + tid, bacc);
   else if (tid < kHid + kOutPad) atomicAdd(a.g_dec + kB2Off + tid - kHid, bacc);
+}
+
+// deterministic mode, after the decoder-backward kernel: the fixed-point accumulator -> the fp32 packed plane gradient (NaN
+// everywhere when the bound or a contribution was not finite), and the per-CTA rows summed in index order in fp64, rounded once
+__global__ void det_planes_kernel(const long long* __restrict__ acc, long long n4, const int* __restrict__ hdr, float* __restrict__ out) {
+  const double inv = ldexp(1.0, -__ldg(hdr));
+  const bool bad = __ldg(hdr + 1) != 0;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
+    const longlong2 u = __ldg(reinterpret_cast<const longlong2*>(acc) + 2 * i), v = __ldg(reinterpret_cast<const longlong2*>(acc) + 2 * i + 1);
+    float4 r = make_float4(__double2float_rn((double)u.x * inv), __double2float_rn((double)u.y * inv),
+                           __double2float_rn((double)v.x * inv), __double2float_rn((double)v.y * inv));
+    if (bad) r = make_float4(__int_as_float(0x7fffffff), __int_as_float(0x7fffffff), __int_as_float(0x7fffffff), __int_as_float(0x7fffffff));
+    reinterpret_cast<float4*>(out)[i] = r;
+  }
+}
+__global__ void det_rows_kernel(const float* __restrict__ rows, int n_rows, float* __restrict__ out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= kDecFloats) return;
+  double sum = 0.0;
+  for (int r = 0; r < n_rows; ++r) sum += (double)__ldg(rows + (size_t)r * kDecFloats + i);
+  out[i] = (float)sum;
 }
 
 // packed decoder gradient -> gradients of the module's raw tensors (training/networks_stylegan2.py:118-127: the runtime gains)
@@ -682,23 +748,49 @@ int launch_bwd_march(const float* dc, const float* df, int Dc, int Df, const flo
   return (int)cudaGetLastError();
 }
 
-// point != 0: point queries (see decode_backward_kernel)
+// point != 0: point queries (see decode_backward_kernel); det != NULL: the deterministic mode, as in launch_bwd_decode_tc
+// (the caller has run launch_det_bound)
 int launch_bwd_decode(const float* planes, int H, int W, const float* dec, const float* pts, const float* colours, int col_chunked,
                       const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total, long long pts_per_img, int S,
-                      int point, float box_scale, float* g_planes, float* g_dec, int fast, int skip, int sms, cudaStream_t st) {
-  bwd::DecArgs a;
+                      int point, float box_scale, float* g_planes, float* g_dec, int fast, int skip, DetScratch* det, int sms, cudaStream_t st) {
+  bwd::DetDecArgs a;
   a.planes = planes; a.H = H; a.W = W; a.dec = dec; a.pts = pts; a.colours = colours; a.col_chunked = col_chunked; a.features = features; a.gsig = gsig; a.omega = omega;
   a.g_rgb = g_rgb; a.total = total; a.pts_per_img = pts_per_img; a.S = S; a.box_scale = box_scale; a.g_planes = g_planes;
   a.g_dec = g_dec;
+  a.g_acc = det ? det->acc : nullptr; a.dec_rows = det ? det->rows : nullptr; a.det_hdr = det ? det->hdr : nullptr;
   { const char* e = getenv("TPR_BWD_DEBUG"); a.debug = skip | (e ? atoi(e) : 0); }
   const size_t smem = sizeof(bwd::Smem) + 16;
-  void (*kern)(const bwd::DecArgs) = point ? (fast ? bwd::decode_backward_kernel<true, true> : bwd::decode_backward_kernel<false, true>)
-                                           : (fast ? bwd::decode_backward_kernel<true, false> : bwd::decode_backward_kernel<false, false>);
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  using bwd::DecArgs; using bwd::DetDecArgs;
+  void (*kern)(const DecArgs) = point ? (fast ? bwd::decode_backward_kernel<true, true> : bwd::decode_backward_kernel<false, true>)
+                                      : (fast ? bwd::decode_backward_kernel<true, false> : bwd::decode_backward_kernel<false, false>);
+  void (*kern_det)(const DetDecArgs) =
+      point ? (fast ? bwd::decode_backward_kernel<true, true, true, DetDecArgs> : bwd::decode_backward_kernel<false, true, true, DetDecArgs>)
+            : (fast ? bwd::decode_backward_kernel<true, false, true, DetDecArgs> : bwd::decode_backward_kernel<false, false, true, DetDecArgs>);
+  cudaError_t e = det ? cudaFuncSetAttribute(kern_det, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                      : cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
   const long long n_tiles = (total + bwd::kT - 1) / bwd::kT;
-  const long long grid = n_tiles < 2 * sms ? n_tiles : 2 * sms;      // two CTAs per SM
+  long long grid = n_tiles < 2 * sms ? n_tiles : 2 * sms;      // two CTAs per SM
+  if (det) {
+    if (grid > kDetMaxRows) grid = kDetMaxRows;
+    det->n_rows = (int)grid;
+    if (!(skip & 2) && (e = cudaMemsetAsync(det->rows, 0, (size_t)grid * kDecFloats * sizeof(float), st)) != cudaSuccess) return (int)e;
+    kern_det<<<(unsigned)grid, bwd::kBT, smem, st>>>(a);
+    return (int)cudaGetLastError();
+  }
   kern<<<(unsigned)grid, bwd::kBT, smem, st>>>(a);
+  return (int)cudaGetLastError();
+}
+
+// deterministic mode: the outputs from det (either output may be NULL)
+int launch_det_finish(const DetScratch* det, long long n_plane_floats, float* g_planes, float* g_dec, int sms, cudaStream_t st) {
+  if (g_planes) {
+    const long long n4 = n_plane_floats / 4;
+    long long blocks = (n4 + 255) / 256;
+    if (blocks > (long long)sms * 16) blocks = (long long)sms * 16;
+    bwd::det_planes_kernel<<<(unsigned)blocks, 256, 0, st>>>(reinterpret_cast<const long long*>(det->acc), n4, det->hdr, g_planes);
+  }
+  if (g_dec) bwd::det_rows_kernel<<<(kDecFloats + 255) / 256, 256, 0, st>>>(det->rows, det->n_rows, g_dec);
   return (int)cudaGetLastError();
 }
 

@@ -34,7 +34,8 @@
 //
 // Roles (25 warps, one CTA per SM):  0-7 LOAD (features / colours / upstream gradient -> operand tiles)
 //                                     8-15 SCATTER (the sample's 12 taps from its position, red.global.add.v4.f32 of GF x tap
-//                                           weight; one texel = one 128-byte line = eight lanes)
+//                                           weight; one texel = one 128-byte line = eight lanes.  kDet: four
+//                                           red.global.add.u64 of the fixed-point value per lane and texel instead)
 //                                     16-23 EPILOGUE (TMEM -> softplus / products -> operand tiles; GF -> shared memory): two
 //                                           warps per TMEM lane quarter, 32 hidden units each
 //                                     24 MMA issuer
@@ -96,6 +97,9 @@ struct Args {
   const float* scale;                   // [2] device: power-of-two scale of the gradient-side operands and its inverse
   int lookahead;                        // G1 + G2 of tile i + 1 ahead of the weight-gradient MMAs of tile i
   long long* prof;                      // TPR_BWD_PROFILE: cycles CTA 0 spends per role and wait (NULL: off)
+  // kDet (deterministic mode): the plane gradient goes to g_acc in fixed point (scale 2^e from det_hdr), the decoder gradient
+  // to this CTA's row of dec_rows; g_planes / g_dec only say whether each is wanted
+  unsigned long long* g_acc; float* dec_rows; int* det_hdr;
 };
 
 // ---- descriptors -------------------------------------------------------------------------------------------------
@@ -184,6 +188,43 @@ __global__ void scale_finish_kernel(const unsigned* __restrict__ acc, const floa
   }
 }
 
+// Deterministic mode: the fixed-point exponent e of the plane-gradient accumulator.  |GF_k| <= max|GA| . sum_j |W1t[k][j]|
+// and |GA| <= |GH| (softplus' <= 1) <= mg wc + ms wsig (the bound of scale_finish_kernel); a texel takes at most K samples'
+// contributions with tap weights of sum <= 1 per plane, so its sum is at most K . bound_GF and e = 62 - ceil(log2(K . bound_GF))
+// cannot overflow.  The bound scales exactly with the upstream gradient, so 2^k x the upstream gradient gives e - k and the
+// same integers.  A non-finite bound (inf upstream) or one whose e would leave the fp32 range marks the result NaN.
+__global__ void det_bound_kernel(const unsigned* __restrict__ acc, const float* __restrict__ dec, long long K, int* __restrict__ hdr) {
+  __shared__ float col[64], row[32];
+  const int j = threadIdx.x;
+  if (j < 64) {
+    float sum = 0.f;
+    for (int c = 0; c < 32; ++c) sum += fabsf(dec[kW2tOff + j * kOutPad + 1 + c]);
+    col[j] = sum;
+  }
+  if (j < 32) {
+    float sum = 0.f;
+    for (int i = 0; i < 64; ++i) sum += fabsf(dec[kW1tOff + j * kHid + i]);
+    row[j] = sum;
+  }
+  __syncthreads();
+  if (j == 0) {
+    const float mg = __uint_as_float(acc[0]) * 0.501f, ms = __uint_as_float(acc[1]);
+    float wc = 0.f, wsig = 0.f, w1 = 0.f;
+    for (int i = 0; i < 64; ++i) { wc = fmaxf(wc, col[i]); wsig = fmaxf(wsig, fabsf(dec[kW2tOff + i * kOutPad])); }
+    for (int k = 0; k < 32; ++k) w1 = fmaxf(w1, row[k]);
+    const double bound = ((double)mg * wc + (double)ms * wsig) * (double)w1 * (double)K;
+    int e = 0, bad = !isfinite(bound);
+    if (!bad && bound > 0.0) {
+      int x;
+      const double m = frexp(bound, &x);       // bound = m 2^x, m in [0.5, 1): ceil(log2(bound)) = x, or x - 1 when m = 0.5
+      e = 62 - (m == 0.5 ? x - 1 : x);
+      if (e < -126) { bad = 1; e = 0; }
+      e = min(e, 127);                         // a tiny bound: 2^127 keeps every contribution far below 2^62
+    }
+    hdr[0] = e; hdr[1] = bad; hdr[2] = __float_as_int(ldexpf(1.0f, e));
+  }
+}
+
 // TPR_BWD_PROFILE=1: CTA 0 adds the cycles each role's first warp spends in every wait / work phase to prof[slot]
 // (kProf instantiation only; accumulated in registers, written once at the end of the role)
 #define PROF_DECL() long long prof_t = 0, prof_acc[17]; if (kProf) { for (int k_ = 0; k_ < 17; ++k_) prof_acc[k_] = 0; }
@@ -191,7 +232,8 @@ __global__ void scale_finish_kernel(const unsigned* __restrict__ acc, const floa
 #define PROF(slot) do { if (kProf) { const long long t1_ = clock64(); prof_acc[slot] += t1_ - prof_t; prof_t = t1_; } } while (0)
 #define PROF_FLUSH(first, last, cond) do { if (kProf && blockIdx.x == 0 && lane == 0 && (cond)) { for (int k_ = first; k_ <= last; ++k_) a.prof[k_] = prof_acc[k_]; } } while (0)
 // ---- the kernel ------------------------------------------------------------------------------------------------------------
-template <bool kProf, bool kPoint>
+// kDet: the deterministic mode (Args::g_acc); the launch then has kLoadWarps x 33 floats of dynamic shared memory past Smem
+template <bool kProf, bool kPoint, bool kDet = false>
 __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const Args a) {
   extern __shared__ uint8_t smem_raw[];
   Smem& s = *reinterpret_cast<Smem*>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
@@ -350,6 +392,7 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
     }
     PROF_FLUSH(0, 3, warp == 0);
     // gb2 (the bias of layer 2): sums of the outputs' gradients
+    if constexpr (!kDet) {
     if (want_dec) {
 #pragma unroll
       for (int j = 0; j < 2; ++j) {
@@ -362,6 +405,31 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
       }
       b2sig = warp_sum(b2sig);
       if (lane == 0) atomicAdd(a.g_dec + kB2Off, b2sig * inv_sc);
+    }
+    } else if (want_dec) {
+      // deterministic: the eight warps' partials meet in shared memory and warp 0 adds them in warp order
+      float* part = reinterpret_cast<float*>(&s + 1);          // [kLoadWarps][33]
+#pragma unroll
+      for (int j = 0; j < 2; ++j) {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+          float v = b2acc[j][k];
+          v += __shfl_xor_sync(kFull, v, 1); v += __shfl_xor_sync(kFull, v, 2); v += __shfl_xor_sync(kFull, v, 4);
+          if (cs == 0) part[warp * 33 + 1 + 4 * (cq + 4 * j) + k] = v;
+        }
+      }
+      b2sig = warp_sum(b2sig);
+      if (lane == 0) part[warp * 33] = b2sig;
+      asm volatile("bar.sync 1, %0;" ::"n"(kLoadWarps * 32) : "memory");
+      if (warp == 0) {
+        float* row = a.dec_rows + (size_t)blockIdx.x * kDecFloats;
+        for (int l = lane; l < 33; l += 32) {
+          float t = 0.f;
+#pragma unroll
+          for (int w = 0; w < kLoadWarps; ++w) t += part[w * 33 + l];
+          row[kB2Off + l] = t * inv_sc;
+        }
+      }
     }
   } else if (warp < kLoadWarps + kScatWarps) {
     // ================================================ SCATTER ================================================
@@ -393,6 +461,29 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
         for (int it = 0; it < 4; ++it) {
           const int sr = sw * 16 + it * 4 + grp;
           if (gs0 + sr < a.total) {
+            if constexpr (kDet) {
+              // deterministic: GF x 2^e, four fixed-point reductions per lane and texel
+              const float fx = __int_as_float(__ldg(a.det_hdr + 2));
+              float4 gf = *reinterpret_cast<const float4*>(s.gf[b] + row_chunk_off(sr, sub));
+              gf = make_float4(gf.x * fx, gf.y * fx, gf.z * fx, gf.w * fx);
+              if (!fixed_ok(gf)) a.det_hdr[1] = 1;
+              const int n = (int)n0 + (rem0 + sr >= a.pts_per_img ? 1 : 0);
+              unsigned long long* img = a.g_acc + (size_t)n * img_stride + sub * 4;
+              const float x = __fmul_rn(px[it], a.box_scale), y = __fmul_rn(py[it], a.box_scale), z = __fmul_rn(pz[it], a.box_scale);
+#pragma unroll
+              for (int p = 0; p < 3; ++p) {
+                Taps tp;
+                plane_taps(p == 2 ? z : x, p == 0 ? y : (p == 1 ? z : x), a.H, a.W, tp);
+#pragma unroll
+                for (int k = 0; k < 4; ++k)
+                  if (tp.w[k] != 0.0f) {
+                    unsigned long long* t = img + (unsigned)(p * plane_stride + tp.off[k]);
+                    red_add_fixed(t, tp.w[k] * gf.x); red_add_fixed(t + 1, tp.w[k] * gf.y);
+                    red_add_fixed(t + 2, tp.w[k] * gf.z); red_add_fixed(t + 3, tp.w[k] * gf.w);
+                  }
+              }
+              continue;
+            }
             const float4 gf = *reinterpret_cast<const float4*>(s.gf[b] + row_chunk_off(sr, sub));
             const int n = (int)n0 + (rem0 + sr >= a.pts_per_img ? 1 : 0);
             float* img = a.g_planes + (size_t)n * img_stride + sub * 4;
@@ -483,6 +574,40 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
     if (want_dec && G > 0) {
       mbar_wait_parked(&s.all_done, 0u);
       tcgen05_fence_after();
+      if constexpr (kDet) {
+      const int j = row & 63;
+      uint32_t v[16], u[16];
+      // every element has one owning thread per CTA: deterministic mode stores it into the CTA's row
+      float* drow = a.dec_rows + (size_t)blockIdx.x * kDecFloats;
+      auto put = [&](int idx, float val) { drow[idx] = val; };
+      if (row < 64) {
+#pragma unroll 1
+        for (int c = hh; c < hh + 1; ++c) {     // x F hi + x F lo: channels k = 16 c ..
+          tmem_ld16(tmem + cW + lane_base + 64 + 16 * c, v);
+          tmem_ld16(tmem + cW + lane_base + 16 * c, u);
+          tmem_wait_ld();
+#pragma unroll
+          for (int k = 0; k < 16; ++k)
+            put(kW1tOff + (16 * c + k) * kHid + j, (__uint_as_float(v[k]) + __uint_as_float(u[k])) * inv_sc);
+        }
+        tmem_ld16(tmem + cW + lane_base + 128, v);
+        tmem_wait_ld();
+        if (hh == 0) put(kB1Off + j, __uint_as_float(v[2]) * inv_sc);        // x the ones column
+      } else {
+#pragma unroll 1
+        for (int c = hh; c < hh + 1; ++c) {
+          tmem_ld16(tmem + cW + lane_base + 96 + 16 * c, v);
+          tmem_ld16(tmem + cW + lane_base + 32 + 16 * c, u);
+          tmem_wait_ld();
+#pragma unroll
+          for (int k = 0; k < 16; ++k)
+            put(kW2tOff + j * kOutPad + 1 + 16 * c + k, (__uint_as_float(v[k]) + __uint_as_float(u[k])) * inv_sc);
+        }
+        tmem_ld16(tmem + cW + lane_base + 128, v);
+        tmem_wait_ld();
+        if (hh == 0) put(kW2tOff + j * kOutPad, (__uint_as_float(v[0]) + __uint_as_float(v[1])) * inv_sc);   // x gsig hi + lo
+      }
+      } else {
       const int j = row & 63;
       uint32_t v[16], u[16];
       if (row < 64) {
@@ -511,6 +636,7 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
         tmem_ld16(tmem + cW + lane_base + 128, v);
         tmem_wait_ld();
         if (hh == 0) atomicAdd(a.g_dec + kW2tOff + j * kOutPad, (__uint_as_float(v[0]) + __uint_as_float(v[1])) * inv_sc);   // x gsig hi + lo
+      }
       }
       tcgen05_fence_before();
     }
@@ -612,34 +738,46 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
 // Launch; returns cudaError_t (0 = ok) or -1 when the device cannot run it (the caller keeps the mma.sync kernel).
 // scale_buf: 4 floats of device scratch ([0..1] the power-of-two scale and its inverse, [2..3] the range accumulators).
 // point != 0: point queries (rows of colours / g_rgb per point, no omega, S unused; g_rgb may be NULL).
+// det != NULL: the deterministic mode (tpr_device.cuh: DetScratch); the launch sets det->n_rows and zeroes those rows, the
+// caller zeroes det->acc and converts both afterwards (launch_det_finish).
 int launch_bwd_decode_tc(const float* planes, int H, int W, const float* dec, const float* pts, const float* colours, int col_chunked,
                          const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total,
                          long long pts_per_img, int S, int point, float box_scale, float* g_planes, float* g_dec, float* scale_buf,
-                         int sms, int smem_optin, cudaStream_t st) {
+                         DetScratch* det, int sms, int smem_optin, cudaStream_t st) {
   using namespace bwdtc;
-  const size_t smem = sizeof(Smem) + 1024;
+  const size_t smem = sizeof(Smem) + 1024 + (det ? kLoadWarps * 33 * sizeof(float) : 0);
   if ((int)smem > smem_optin) return -1;
   cudaError_t e = cudaMemsetAsync(scale_buf + 2, 0, 2 * sizeof(float), st);
   if (e != cudaSuccess) return (int)e;
   const long long n_rgb = point ? (g_rgb ? total * 32 : 0) : (total / S) * 32;
   scale_kernel<<<sms * 4, 256, 0, st>>>(g_rgb, n_rgb, gsig, total, dec, reinterpret_cast<unsigned*>(scale_buf + 2));
   scale_finish_kernel<<<1, 64, 0, st>>>(reinterpret_cast<const unsigned*>(scale_buf + 2), dec, scale_buf);
+  if (det) det_bound_kernel<<<1, 64, 0, st>>>(reinterpret_cast<const unsigned*>(scale_buf + 2), dec, pts_per_img, det->hdr);
   Args a;
   a.planes = planes; a.H = H; a.W = W; a.dec = dec; a.pts = pts; a.colours = colours; a.col_chunked = col_chunked; a.features = features; a.gsig = gsig;
   a.omega = omega; a.g_rgb = g_rgb; a.total = total; a.pts_per_img = pts_per_img; a.S = S; a.box_scale = box_scale;
   a.g_planes = g_planes; a.g_dec = g_dec; a.scale = scale_buf; a.prof = nullptr;
+  a.g_acc = det ? det->acc : nullptr; a.dec_rows = det ? det->rows : nullptr; a.det_hdr = det ? det->hdr : nullptr;
   { const char* dbg = getenv("TPR_BWD_DEBUG"); const int d = dbg ? atoi(dbg) : 0;      // profiling A/B: 1 = no scatter, 2 = no weight gradients
     if (d & 1) a.g_planes = nullptr;
     if (d & 2) a.g_dec = nullptr;
     a.lookahead = (d & 8) ? 0 : 1; }
   static const bool profile = getenv("TPR_BWD_PROFILE") != nullptr;
-  void (*kern)(const Args) = profile ? (point ? decode_backward_tc_kernel<true, true> : decode_backward_tc_kernel<true, false>)
+  void (*kern)(const Args) = det ? (point ? decode_backward_tc_kernel<false, true, true> : decode_backward_tc_kernel<false, false, true>)
+                           : profile ? (point ? decode_backward_tc_kernel<true, true> : decode_backward_tc_kernel<true, false>)
                                      : (point ? decode_backward_tc_kernel<false, true> : decode_backward_tc_kernel<false, false>);
   e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
   if (pts_per_img < kM) return -1;                 // (a tile may straddle at most two images)
   const long long n_tiles = (total + kM - 1) / kM;
-  const long long grid = n_tiles < sms ? n_tiles : sms;
+  long long grid = n_tiles < sms ? n_tiles : sms;
+  if (det) {
+    if (grid > kDetMaxRows) grid = kDetMaxRows;
+    det->n_rows = (int)grid;
+    if (g_dec && (e = cudaMemsetAsync(det->rows, 0, (size_t)grid * kDecFloats * sizeof(float), st)) != cudaSuccess) return (int)e;
+    kern<<<(unsigned)grid, kThreads, smem, st>>>(a);
+    return (int)cudaGetLastError();
+  }
   if (profile) {                                    // debugging aid: synchronous, prints CTA 0's cycles per role and phase
     static const char* names[17] = {"load: issue loads", "-", "load: wait in_free", "load: operands", "scatter: load points",
                                     "scatter: wait gf_ready", "scatter: red", "epi: wait g12_done", "epi: wait wg_done", "epi: H/GA",
@@ -656,6 +794,19 @@ int launch_bwd_decode_tc(const float* planes, int H, int W, const float* dec, co
     return (int)cudaGetLastError();
   }
   kern<<<(unsigned)grid, kThreads, smem, st>>>(a);
+  return (int)cudaGetLastError();
+}
+
+// Deterministic mode ahead of the mma.sync kernel: the upstream gradient's range and the fixed-point exponent into det->hdr
+// (what launch_bwd_decode_tc computes on its way).  Arguments as there.
+int launch_det_bound(const float* dec, const float* gsig, const float* g_rgb, long long total, long long pts_per_img, int S, int point,
+                     float* scale_buf, DetScratch* det, int sms, cudaStream_t st) {
+  using namespace bwdtc;
+  cudaError_t e = cudaMemsetAsync(scale_buf + 2, 0, 2 * sizeof(float), st);
+  if (e != cudaSuccess) return (int)e;
+  const long long n_rgb = point ? (g_rgb ? total * 32 : 0) : (total / S) * 32;
+  scale_kernel<<<sms * 4, 256, 0, st>>>(g_rgb, n_rgb, gsig, total, dec, reinterpret_cast<unsigned*>(scale_buf + 2));
+  det_bound_kernel<<<1, 64, 0, st>>>(reinterpret_cast<const unsigned*>(scale_buf + 2), dec, pts_per_img, det->hdr);
   return (int)cudaGetLastError();
 }
 

@@ -27,6 +27,33 @@ static_assert(kDecFloats % 4 == 0, "decoder block must be float4 copyable");
 constexpr unsigned kFull = 0xffffffffu;
 
 // ---------------------------------------------------------------------------------------
+// deterministic backward (TPR_BWD_DETERMINISTIC): the scratch the decoder-backward kernels use in that mode
+// ---------------------------------------------------------------------------------------
+// The plane gradient is accumulated in fixed point: every contribution is scaled by 2^e (e from a bound on any texel's sum,
+// so nothing overflows 2^62), rounded to int64 and added with integer reductions -- associative, so the result does not
+// depend on the order of the samples.  The decoder gradient: every CTA stores its partial sums as one row, and the rows are
+// summed in index order.  A launch clamps its grid to kDetMaxRows CTAs.
+constexpr int kDetMaxRows = 512;
+struct DetScratch {
+  int* hdr;                    // [0] e, [1] non-zero: non-finite bound or contribution (the plane gradient becomes NaN),
+                               // [2] the bits of the fp32 2^e
+  float* rows;                 // [kDetMaxRows][kDecFloats] per-CTA decoder-gradient rows
+  unsigned long long* acc;     // [N,3,H,W,32] fixed-point plane gradient (two's complement), zero-initialised
+  int n_rows;                  // (host) rows the launch wrote
+};
+
+// one fixed-point contribution: v (already x 2^e) rounded to the nearest integer, added as a two's-complement u64
+__device__ __forceinline__ void red_add_fixed(unsigned long long* p, float v) {
+  long long q;
+  asm("cvt.rni.s64.f32 %0, %1;" : "=l"(q) : "f"(v));
+  asm volatile("red.global.add.u64 [%0], %1;" ::"l"(p), "l"(q) : "memory");
+}
+// false for NaN, +-inf and magnitudes the int64 accumulator cannot take
+__device__ __forceinline__ bool fixed_ok(float4 v) {
+  return fabsf(v.x) < 0x1p62f && fabsf(v.y) < 0x1p62f && fabsf(v.z) < 0x1p62f && fabsf(v.w) < 0x1p62f;
+}
+
+// ---------------------------------------------------------------------------------------
 // scalar math
 // ---------------------------------------------------------------------------------------
 // torch.nn.Softplus(beta=1, threshold=20): log1p(exp(x)), identity above the threshold.

@@ -34,12 +34,16 @@ int launch_bwd_march(const float* dc, const float* df, int Dc, int Df, const flo
                      long long n_rays_total, float* gsig, float* omega, int sms, cudaStream_t st);
 int launch_bwd_decode(const float* planes, int H, int W, const float* dec, const float* pts, const float* colours, int col_chunked,
                       const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total, long long pts_per_img, int S,
-                      int point, float box_scale, float* g_planes, float* g_dec, int fast, int skip, int sms, cudaStream_t st);
+                      int point, float box_scale, float* g_planes, float* g_dec, int fast, int skip, DetScratch* det, int sms,
+                      cudaStream_t st);
+int launch_det_finish(const DetScratch* det, long long n_plane_floats, float* g_planes, float* g_dec, int sms, cudaStream_t st);
 // tpr_backward_tc.cu: the decoder backward on tcgen05 (returns -1 if it cannot run here)
 int launch_bwd_decode_tc(const float* planes, int H, int W, const float* dec, const float* pts, const float* colours, int col_chunked,
                          const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total,
                          long long pts_per_img, int S, int point, float box_scale, float* g_planes, float* g_dec, float* scale_buf,
-                         int sms, int smem_optin, cudaStream_t st);
+                         DetScratch* det, int sms, int smem_optin, cudaStream_t st);
+int launch_det_bound(const float* dec, const float* gsig, const float* g_rgb, long long total, long long pts_per_img, int S, int point,
+                     float* scale_buf, DetScratch* det, int sms, cudaStream_t st);
 int launch_unpack_decoder_grad(const float* gd, float g_w1, float g_b1, float g_w2, float g_b2, float* w1, float* b1, float* w2,
                                float* b2, cudaStream_t st);
 
@@ -1254,6 +1258,62 @@ size_t tpr_render_backward_scratch_bytes(int64_t n_img, int64_t n_rays, int32_t 
   return align256(T * 12) + align256(T * 128) + 3 * align256(T * 4) + 256;
 }
 
+// TPR_BWD_DETERMINISTIC: [256 B: DetScratch::hdr][kDetMaxRows decoder rows][int64 accumulator [N,3,H,W,32]]
+size_t tpr_backward_deterministic_scratch_bytes(int64_t n_img, int32_t height, int32_t width) {
+  if (n_img <= 0 || height <= 0 || width <= 0) return 0;
+  return 256 + align256((size_t)kDetMaxRows * kDecFloats * sizeof(float)) +
+         align256((size_t)n_img * 3 * (size_t)height * (size_t)width * kC * sizeof(long long));
+}
+static DetScratch det_scratch(void* scratch, size_t base) {
+  uint8_t* q = (uint8_t*)scratch + base;
+  DetScratch d;
+  d.hdr = (int*)q; q += 256;
+  d.rows = (float*)q; q += align256((size_t)kDetMaxRows * kDecFloats * sizeof(float));
+  d.acc = (unsigned long long*)q;
+  d.n_rows = 0;
+  return d;
+}
+
+// The decoder backward of both entry points: tcgen05 + TMEM, warp-specialised (tpr_backward_tc.cu) first; the mma.sync kernel
+// when it refuses (fewer than 128 samples per image, too little shared memory) or with TPR_BWD_IMPL=hmma (A/B runs).  The outputs
+// are zeroed here.  det != NULL: the deterministic mode, its outputs converted after the kernel.
+static int decoder_backward(const float* planes_packed, int64_t n_img, int32_t height, int32_t width, const float* dec, const float* pts,
+                            const float* colours, int col_chunked, const float* features, const float* gsig, const float* omega,
+                            const float* g_rgb, long long total, long long pts_per_img, int S, int point, float box_scale, int fast,
+                            float* g_planes_packed, float* g_decoder_packed, float* scale_buf, void* scratch, DetScratch* det,
+                            const DeviceInfo& di, cudaStream_t st) {
+  const size_t plane_floats = (size_t)n_img * 3 * height * width * kC;
+  cudaError_t e = cudaSuccess;
+  if (g_planes_packed) e = det ? cudaMemsetAsync(det->acc, 0, plane_floats * sizeof(long long), st)
+                               : cudaMemsetAsync(g_planes_packed, 0, plane_floats * sizeof(float), st);
+  if (e == cudaSuccess && g_decoder_packed && !det) e = cudaMemsetAsync(g_decoder_packed, 0, kDecFloats * sizeof(float), st);
+  if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync");
+  const char* impl = getenv("TPR_BWD_IMPL");
+  int rc = -1;
+  if (!(impl && strcmp(impl, "hmma") == 0)) {
+    rc = launch_bwd_decode_tc(planes_packed, height, width, dec, pts, colours, col_chunked, features, gsig, omega, g_rgb, total,
+                              pts_per_img, S, point, box_scale, g_planes_packed, g_decoder_packed, scale_buf, det, di.sms,
+                              di.smem_optin, st);
+    if (rc > 0) return cuda_fail((cudaError_t)rc, "decode_backward_tc_kernel");
+  }
+  if (rc != 0) {
+    if (det) {
+      rc = launch_det_bound(dec, gsig, g_rgb, total, pts_per_img, S, point, scale_buf, det, di.sms, st);
+      if (rc != 0) return cuda_fail((cudaError_t)rc, "det_bound_kernel");
+    }
+    float* g_dec_out = g_decoder_packed ? g_decoder_packed : reinterpret_cast<float*>(scratch);      // (never written when skipped)
+    rc = launch_bwd_decode(planes_packed, height, width, dec, pts, colours, col_chunked, features, gsig, omega, g_rgb, total,
+                           pts_per_img, S, point, box_scale, g_planes_packed, g_dec_out, fast,
+                           (g_planes_packed ? 0 : 1) | (g_decoder_packed ? 0 : 2), det, di.sms, st);
+    if (rc != 0) return cuda_fail((cudaError_t)rc, "decode_backward_kernel");
+  }
+  if (det) {
+    rc = launch_det_finish(det, (long long)plane_floats, g_planes_packed, g_decoder_packed, di.sms, st);
+    if (rc != 0) return cuda_fail((cudaError_t)rc, "det_planes_kernel");
+  }
+  return 0;
+}
+
 int tpr_march_backward(const float* depths_coarse, const float* depths_fine, int32_t dc, int32_t df, const float* sigma,
                        const float* colours, const float* g_rgb, const float* g_depth, const float* g_weight_sum,
                        const float* depth_range, int32_t white_back, int64_t n_rays_total, float* g_sigma, float* omega,
@@ -1288,7 +1348,13 @@ int tpr_render_backward(const float* planes_packed, int64_t n_img, int32_t heigh
   if (opt->plane_sets != 0 && opt->plane_sets != n_img) return fail(TPR_E_OPTION, "tpr_render_backward: one plane set per image only");
   if (opt->depth_clamp_group != 0) return fail(TPR_E_OPTION, "tpr_render_backward: depth_clamp_group is not supported");
   if (!(opt->box_warp > 0)) return fail(TPR_E_OPTION, "tpr_render_backward: box_warp must be > 0");
-  if (scratch_bytes < tpr_render_backward_scratch_bytes(n_img, n_rays, S)) return fail(TPR_E_SCRATCH, "tpr_render_backward: scratch too small");
+  const bool det = (opt->flags & TPR_BWD_DETERMINISTIC) != 0;
+  const int32_t mlp = opt->flags & ~TPR_BWD_DETERMINISTIC;
+  if (mlp != TPR_MLP_FP32 && mlp != TPR_MLP_BF16 && mlp != TPR_MLP_FFMA)
+    return fail(TPR_E_OPTION, "tpr_render_backward: unknown flag");
+  const size_t base_bytes = tpr_render_backward_scratch_bytes(n_img, n_rays, S);
+  if (scratch_bytes < base_bytes + (det ? tpr_backward_deterministic_scratch_bytes(n_img, height, width) : 0))
+    return fail(TPR_E_SCRATCH, "tpr_render_backward: scratch too small");
   DeviceInfo di = device_info();
   if (!di.ok) return fail(TPR_E_DEVICE, "tpr_render_backward: no CUDA device");
   cudaStream_t st = (cudaStream_t)stream;
@@ -1309,33 +1375,17 @@ int tpr_render_backward(const float* planes_packed, int64_t n_img, int32_t heigh
     // not kept by the forward (tpr_render_train): colours and densities of every sample through the forward's point query
     // (VR/renderer.py:142-148)
     rc = tpr_run_model(planes_packed, n_img, height, width, decoder_packed, pts, (int64_t)n_rays * S, opt->box_warp, colours, sigma,
-                       opt->flags, stream);
+                       mlp, stream);
     if (rc != 0) return rc;
     col_in = colours; sig_in = sigma;
   }
   rc = launch_bwd_march(depths_coarse, depths_fine, Dc, Df, sig_in, col_in, col_chunked, g_rgb, g_depth, g_weight_sum, depth_range,
                         opt->white_back, rays, gsig, omega, di.sms, st);
   if (rc != 0) return cuda_fail((cudaError_t)rc, "march_backward_kernel");
-  cudaError_t e = cudaSuccess;
-  if (g_planes_packed) e = cudaMemsetAsync(g_planes_packed, 0, (size_t)n_img * 3 * height * width * kC * sizeof(float), st);
-  if (e == cudaSuccess && g_decoder_packed) e = cudaMemsetAsync(g_decoder_packed, 0, kDecFloats * sizeof(float), st);
-  if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync");
-  // The decoder backward: tcgen05 + TMEM, warp-specialised (tpr_backward_tc.cu).  TPR_BWD_IMPL=hmma selects the mma.sync kernel
-  // it replaced (A/B runs; also the fallback if the tcgen05 kernel's shared memory does not fit the device).
-  const char* impl = getenv("TPR_BWD_IMPL");
-  if (!(impl && strcmp(impl, "hmma") == 0)) {
-    rc = launch_bwd_decode_tc(planes_packed, height, width, decoder_packed, pts, col_in, col_chunked, sample_features, gsig, omega, g_rgb, (long long)T,
-                              (long long)n_rays * S, S, 0, (float)(2.0 / opt->box_warp), g_planes_packed, g_decoder_packed, scale_buf,
-                              di.sms, di.smem_optin, st);
-    if (rc > 0) return cuda_fail((cudaError_t)rc, "decode_backward_tc_kernel");
-    if (rc == 0) return 0;
-  }
-  float* g_dec_out = g_decoder_packed ? g_decoder_packed : reinterpret_cast<float*>(scratch);      // (never written when skipped)
-  rc = launch_bwd_decode(planes_packed, height, width, decoder_packed, pts, col_in, col_chunked, sample_features, gsig, omega, g_rgb, (long long)T,
-                         (long long)n_rays * S, S, 0, (float)(2.0 / opt->box_warp), g_planes_packed, g_dec_out,
-                         opt->flags == TPR_MLP_BF16, (g_planes_packed ? 0 : 1) | (g_decoder_packed ? 0 : 2), di.sms, st);
-  if (rc != 0) return cuda_fail((cudaError_t)rc, "decode_backward_kernel");
-  return 0;
+  DetScratch ds = det_scratch(scratch, base_bytes);
+  return decoder_backward(planes_packed, n_img, height, width, decoder_packed, pts, col_in, col_chunked, sample_features, gsig, omega,
+                          g_rgb, (long long)T, (long long)n_rays * S, S, 0, (float)(2.0 / opt->box_warp), mlp == TPR_MLP_BF16,
+                          g_planes_packed, g_decoder_packed, scale_buf, scratch, det ? &ds : nullptr, di, st);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1359,9 +1409,12 @@ int tpr_run_model_backward(const float* planes_packed, int64_t n_img, int32_t he
   if (n_img <= 0 || n_pts <= 0 || height <= 0 || width <= 0) return fail(TPR_E_SHAPE, "tpr_run_model_backward: bad shape");
   if ((long long)3 * height * width * kC >= (1ll << 32)) return fail(TPR_E_SHAPE, "tpr_run_model_backward: planes too large");
   if (!(box_warp > 0)) return fail(TPR_E_OPTION, "tpr_run_model_backward: box_warp must be > 0");
+  const bool det = (flags & TPR_BWD_DETERMINISTIC) != 0;
+  flags &= ~TPR_BWD_DETERMINISTIC;
   if (flags != TPR_MLP_FP32 && flags != TPR_MLP_BF16 && flags != TPR_MLP_FFMA)
     return fail(TPR_E_OPTION, "tpr_run_model_backward: unknown decoder flag");
-  if (scratch_bytes < tpr_run_model_backward_scratch_bytes(n_img, n_pts))
+  const size_t base_bytes = tpr_run_model_backward_scratch_bytes(n_img, n_pts);
+  if (scratch_bytes < base_bytes + (det ? tpr_backward_deterministic_scratch_bytes(n_img, height, width) : 0))
     return fail(TPR_E_SCRATCH, "tpr_run_model_backward: scratch too small");
   DeviceInfo di = device_info();
   if (!di.ok) return fail(TPR_E_DEVICE, "tpr_run_model_backward: no CUDA device");
@@ -1369,29 +1422,16 @@ int tpr_run_model_backward(const float* planes_packed, int64_t n_img, int32_t he
   const long long T = (long long)n_img * n_pts;
   float* zero_gsig = (float*)scratch;
   float* scale_buf = (float*)((uint8_t*)scratch + align256((size_t)T * 4));
-  cudaError_t e = cudaSuccess;
-  if (!g_sigma) e = cudaMemsetAsync(zero_gsig, 0, (size_t)T * sizeof(float), st);
-  if (e == cudaSuccess && g_planes_packed) e = cudaMemsetAsync(g_planes_packed, 0, (size_t)n_img * 3 * height * width * kC * sizeof(float), st);
-  if (e == cudaSuccess && g_decoder_packed) e = cudaMemsetAsync(g_decoder_packed, 0, kDecFloats * sizeof(float), st);
-  if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync");
+  if (!g_sigma) {
+    const cudaError_t e = cudaMemsetAsync(zero_gsig, 0, (size_t)T * sizeof(float), st);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync");
+  }
   const float* gsig = g_sigma ? g_sigma : zero_gsig;
   const float box_scale = (float)(2.0 / box_warp);      // python float (VR/renderer.py:61)
-  // tcgen05 first, the mma.sync kernel when it refuses (fewer than 128 points per image, too little shared memory) or with
-  // TPR_BWD_IMPL=hmma -- as in tpr_render_backward
-  const char* impl = getenv("TPR_BWD_IMPL");
-  int rc;
-  if (!(impl && strcmp(impl, "hmma") == 0)) {
-    rc = launch_bwd_decode_tc(planes_packed, height, width, decoder_packed, xyz, rgb, 0, nullptr, gsig, nullptr, g_rgb, T, n_pts, 1, 1,
-                              box_scale, g_planes_packed, g_decoder_packed, scale_buf, di.sms, di.smem_optin, st);
-    if (rc > 0) return cuda_fail((cudaError_t)rc, "decode_backward_tc_kernel");
-    if (rc == 0) return 0;
-  }
-  float* g_dec_out = g_decoder_packed ? g_decoder_packed : reinterpret_cast<float*>(scratch);      // (never written when skipped)
-  rc = launch_bwd_decode(planes_packed, height, width, decoder_packed, xyz, rgb, 0, nullptr, gsig, nullptr, g_rgb, T, n_pts, 1, 1,
-                         box_scale, g_planes_packed, g_dec_out, flags == TPR_MLP_BF16, (g_planes_packed ? 0 : 1) | (g_decoder_packed ? 0 : 2),
-                         di.sms, st);
-  if (rc != 0) return cuda_fail((cudaError_t)rc, "decode_backward_kernel");
-  return 0;
+  DetScratch ds = det_scratch(scratch, base_bytes);
+  return decoder_backward(planes_packed, n_img, height, width, decoder_packed, xyz, rgb, 0, nullptr, gsig, nullptr, g_rgb, T, n_pts, 1, 1,
+                          box_scale, flags == TPR_MLP_BF16, g_planes_packed, g_decoder_packed, scale_buf, scratch, det ? &ds : nullptr,
+                          di, st);
 }
 
 int tpr_unpack_decoder_grad(const float* g_decoder_packed, float w1_gain, float b1_gain, float w2_gain, float b2_gain, float* g_w1,

@@ -10,6 +10,10 @@ way -- the 32 colours and sigma of every sample (132 B per sample; eager autogra
 
 The graph is the reference's: importance depths are constants (VR/renderer.py:198,210: no_grad + detach), so is the
 jitter; ray origins / directions are not differentiated (they raise if they require grad).
+
+Under ``torch.use_deterministic_algorithms(True)`` both backward functions run the library's deterministic backward
+(TPR_BWD_DETERMINISTIC): bit-identical gradients for equal inputs on the same GPU model, and a plane gradient that does not
+depend on the order of the samples.  The forward is deterministic in either mode.
 """
 import ctypes
 
@@ -59,9 +63,12 @@ class _Render(torch.autograd.Function):
             g_planes = torch.empty_like(packed) if want_planes else None
             g_dec = torch.empty_like(dec) if want_dec else None
             nbytes = L.tpr_render_backward_scratch_bytes(n, m, o.depth_resolution + o.depth_resolution_importance)
-            scratch = torch.empty(nbytes, device=dev, dtype=torch.uint8)
             o2 = _lib.TprOptions.from_buffer_copy(o)
             o2.plane_sets, o2.depth_clamp_group = 0, 0
+            if torch.are_deterministic_algorithms_enabled():
+                o2.flags |= _lib.BWD_DETERMINISTIC
+                nbytes += L.tpr_backward_deterministic_scratch_bytes(n, pp.height, pp.width)
+            scratch = torch.empty(nbytes, device=dev, dtype=torch.uint8)
             _lib.check(L.tpr_render_backward(p(packed), n, pp.height, pp.width, p(dec), p(origins), p(dirs), m, p(coarse),
                                              p(fine) if ctx.has_fine else None, p(rng), ctypes.byref(o2), p(g_rgb), p(g_depth),
                                              p(g_wsum), p(s_col) if ctx.has_saved else None, p(s_sig) if ctx.has_saved else None,
@@ -150,9 +157,13 @@ class _RunModel(torch.autograd.Function):
             g_planes = torch.empty_like(packed) if want_planes else None
             g_dec = torch.empty_like(dec) if want_dec else None
             nbytes = L.tpr_run_model_backward_scratch_bytes(n, npts)
+            flags = ctx.flags
+            if torch.are_deterministic_algorithms_enabled():
+                flags |= _lib.BWD_DETERMINISTIC
+                nbytes += L.tpr_backward_deterministic_scratch_bytes(n, pp.height, pp.width)
             scratch = torch.empty(nbytes, device=dev, dtype=torch.uint8)
             _lib.check(L.tpr_run_model_backward(p(packed), n, pp.height, pp.width, p(dec), p(xyz), npts, ctx.box_warp,
-                                                p(rgb) if g_rgb is not None else None, p(g_rgb), p(g_sigma), ctx.flags,
+                                                p(rgb) if g_rgb is not None else None, p(g_rgb), p(g_sigma), flags,
                                                 p(g_planes), p(g_dec), p(scratch), nbytes, st()),
                        'tpr_run_model_backward')
             g_nchw, g_w1, g_b1, g_w2, g_b2 = _unpack_grads(g_planes, g_dec, ctx.gains, pp, dev)

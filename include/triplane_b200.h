@@ -56,6 +56,13 @@ enum {
   TPR_MLP_BF16 = 1,     /* decoder on tensor cores with bf16 operands: the >= 50 dB PSNR mode */
   TPR_MLP_FFMA = 2      /* force the fp32 FFMA kernel (A/B comparisons) */
 };
+/* A bit OR-ed into the flags of tpr_render_backward (opt->flags) and tpr_run_model_backward (flags): the deterministic
+ * backward.  Two calls with equal inputs on the same device give bit-identical gradients, and the plane gradient does not
+ * depend on the order of the samples: it is accumulated in 64-bit fixed point (every contribution scaled by a power of two
+ * chosen from a bound on any texel's sum, so nothing overflows).  The decoder gradient is summed per CTA and the partial
+ * rows are added in a fixed order in fp64: bit-identical for the same GPU model and shape, not across GPUs with different
+ * SM counts.  Needs tpr_backward_deterministic_scratch_bytes more scratch.  The forward is deterministic without it. */
+#define TPR_BWD_DETERMINISTIC 0x100
 
 /* The subset of `rendering_options` the hot path reads (SURVEY.md section 5, option table;
  * VR/renderer.py:91-100,116,143-146; VR/ray_marcher.py:32,52). */
@@ -341,6 +348,10 @@ int tpr_run_model_backward(const float* planes_packed, int64_t n_img, int32_t he
                            const float* g_sigma /*[N,P] or NULL*/, int32_t flags,
                            float* g_planes_packed /*or NULL*/, float* g_decoder_packed /*or NULL*/,
                            void* scratch, size_t scratch_bytes, void* stream);
+/* Extra scratch of the deterministic backward (TPR_BWD_DETERMINISTIC), on top of tpr_render_backward_scratch_bytes /
+ * tpr_run_model_backward_scratch_bytes: the int64 plane-gradient accumulator [N,3,H,W,32] plus 512 per-CTA rows of the
+ * packed decoder gradient (a launch in this mode uses at most 512 CTAs) and 256 bytes.  0 for a bad shape. */
+size_t tpr_backward_deterministic_scratch_bytes(int64_t n_img, int32_t height, int32_t width);
 /* the two stages of tpr_render_backward, stand-alone (tests): the march's backward -- sigma [R,S], colours [R,S,32] of
  * the samples in forward order -> g_sigma [R,S] and the composite weight omega [R,S] of each sample's colour
  * (dL/d(colour_c) = 2 * g_rgb_c * omega) */
