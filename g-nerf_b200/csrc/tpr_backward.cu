@@ -62,7 +62,9 @@ struct MarchArgs {
   const float* g_rgb;            // [rays, 32]
   const float* g_depth;          // [rays]
   const float* g_wsum;           // [rays]
-  const float* range;            // [2]: the forward's (min, max) of all depths (VR/ray_marcher.py:50)
+  const float* range;            // [2]: the forward's (min, max) of all depths (VR/ray_marcher.py:50); group_rays > 0: one pair
+                                 // per group of group_rays consecutive rays (tpr_render's depth_clamp_group), ray g reads pair g / group_rays
+  unsigned group_rays;           // <= the rays of the call, which tpr_render_backward bounds below 2^32 when group_rays > 0
   int white_back;
   long long n_rays;
   float* gsig;                   // [rays, S]   d(loss)/d(sigma), sample order
@@ -88,7 +90,7 @@ __global__ void __launch_bounds__(128, 8) march_backward_kernel(const MarchArgs 
   float* a2s = sm + 4 * 7 * S + wid * 32;          // 2 x the ray's upstream rgb gradient (shared memory: 32 registers less per
                                                    // thread = 10 instead of 6 resident CTAs, and the kernel waits for DRAM)
   const bool vec = (S & 3) == 0 && (a.Dc & 3) == 0; // float4 reads of the depth rows are aligned
-  const float lo = __ldg(a.range), hi = __ldg(a.range + 1);
+  const float glo = __ldg(a.range), ghi = __ldg(a.range + 1);
   for (long long g = blockIdx.x * 4ll + wid; g < a.n_rays; g += gridDim.x * 4ll) {
     // upstream gradient of rgb (x2: VR/ray_marcher.py:55)
     float sumA2 = 0.0f;
@@ -209,7 +211,10 @@ __global__ void __launch_bounds__(128, 8) march_backward_kernel(const MarchArgs 
     }
     wsum = warp_sum(wsum); dnum = warp_sum(dnum);
     const float depth_raw = dnum / wsum;
-    // nan_to_num + clamp (VR/ray_marcher.py:49-50): the gradient passes only where the depth is inside the range
+    // nan_to_num + clamp (VR/ray_marcher.py:49-50): the gradient passes only where the depth is inside the range (of the ray's
+    // clamp group, group_rays > 0)
+    float lo = glo, hi = ghi;
+    if (a.group_rays > 0) { const unsigned j = (unsigned)g / a.group_rays; lo = __ldg(a.range + 2 * j); hi = __ldg(a.range + 2 * j + 1); }
     const bool pass = depth_raw >= lo && depth_raw <= hi;
     const float bscale = pass ? B / wsum : 0.0f;
     const float wb = a.white_back ? sumA2 : 0.0f;               // rgb += 1 - sum(w) (VR/ray_marcher.py:52-53)
@@ -267,11 +272,11 @@ struct __align__(16) Smem {
   float GF[kT * FS];                    // d/d(features)
   uint32_t tap_off[kT * 12];            // float offset of each tap's texel inside its image
   float tap_w[kT * 12];
-  int simg[kT];
+  int simg[kT];                         // the plane set of each sample
 };
 
 struct DecArgs {
-  const float* planes; int H, W;        // packed [N,3,H,W,32]
+  const float* planes; int H, W;        // packed [P,3,H,W,32]: image n samples plane set n % n_sets
   const float* dec;                     // packed decoder
   const float* pts;                     // [T,3]
   const float* colours;                 // [T,32], or (col_chunked != 0) [rays, 8, S, 4]
@@ -285,6 +290,7 @@ struct DecArgs {
   float* g_dec;                         // [kDecFloats], zero-initialised
   int debug;                            // bit 0: no plane-gradient scatter, bit 1: no weight-gradient phase (the caller does not want
                                         // that gradient; TPR_BWD_DEBUG ORs into it for profiling A/B runs)
+  int n_sets;                           // plane sets in planes / g_planes
 };
 // DET (deterministic mode): the plane gradient goes to g_acc in fixed point (scale 2^e from det_hdr), the decoder gradient to
 // this CTA's row of dec_rows (a separate type, so that the default kernels' parameter block stays as it is)
@@ -356,6 +362,7 @@ __global__ void __launch_bounds__(kBT, 2) decode_backward_kernel(const Args a) {
   for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
     const long long gs0 = tile * kT;
     const long long n0 = gs0 / a.pts_per_img, rem0 = gs0 - n0 * a.pts_per_img;
+    const int set0 = POINT ? (int)n0 : (int)n0 % a.n_sets;      // the plane set of the tile's first image (point queries: n_sets = n_img)
     const long long ray0 = POINT ? 0 : gs0 / a.S;
     const int rr0 = POINT ? 0 : (int)(gs0 - ray0 * a.S);
     // ---- taps of this warp's 8 samples x 3 planes (VR/renderer.py:39-65)
@@ -368,8 +375,8 @@ __global__ void __launch_bounds__(kBT, 2) decode_backward_kernel(const Args a) {
         const float px = __fmul_rn(__ldg(a.pts + 3 * gs + 0), a.box_scale), py = __fmul_rn(__ldg(a.pts + 3 * gs + 1), a.box_scale),
                     pz = __fmul_rn(__ldg(a.pts + 3 * gs + 2), a.box_scale);
         plane_taps(p == 2 ? pz : px, p == 0 ? py : (p == 1 ? pz : px), a.H, a.W, tp);      // (x,y) (x,z) (z,x)
-        long long r = rem0 + sr; n = (int)n0;
-        while (r >= a.pts_per_img) { r -= a.pts_per_img; ++n; }
+        long long r = rem0 + sr; n = set0;
+        while (r >= a.pts_per_img) { r -= a.pts_per_img; if (++n == a.n_sets && !POINT) n = 0; }
       } else {
 #pragma unroll
         for (int k = 0; k < 4; ++k) { tp.off[k] = 0; tp.w[k] = 0.0f; }
@@ -729,11 +736,11 @@ int launch_bwd_points(const float* origins, const float* dirs, const float* dc, 
 }
 
 int launch_bwd_march(const float* dc, const float* df, int Dc, int Df, const float* sigma, const float* colours, int col_chunked,
-                     const float* g_rgb, const float* g_depth, const float* g_wsum, const float* range, int white_back,
-                     long long n_rays_total, float* gsig, float* omega, int sms, cudaStream_t st) {
+                     const float* g_rgb, const float* g_depth, const float* g_wsum, const float* range, long long group_rays,
+                     int white_back, long long n_rays_total, float* gsig, float* omega, int sms, cudaStream_t st) {
   bwd::MarchArgs a;
   a.dc = dc; a.df = df; a.Dc = Dc; a.Df = Df; a.sigma = sigma; a.colours = colours; a.chunked = col_chunked; a.g_rgb = g_rgb; a.g_depth = g_depth;
-  a.g_wsum = g_wsum; a.range = range; a.white_back = white_back; a.n_rays = n_rays_total; a.gsig = gsig; a.omega = omega;
+  a.g_wsum = g_wsum; a.range = range; a.group_rays = (unsigned)group_rays; a.white_back = white_back; a.n_rays = n_rays_total; a.gsig = gsig; a.omega = omega;
   const int S = Dc + Df;
   const size_t smem = (size_t)4 * (7 * S + 32) * sizeof(float);
   long long blocks = (n_rays_total + 3) / 4;
@@ -751,10 +758,11 @@ int launch_bwd_march(const float* dc, const float* df, int Dc, int Df, const flo
 // point != 0: point queries (see decode_backward_kernel); det != NULL: the deterministic mode, as in launch_bwd_decode_tc
 // (the caller has run launch_det_bound)
 int launch_bwd_decode(const float* planes, int H, int W, const float* dec, const float* pts, const float* colours, int col_chunked,
-                      const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total, long long pts_per_img, int S,
-                      int point, float box_scale, float* g_planes, float* g_dec, int fast, int skip, DetScratch* det, int sms, cudaStream_t st) {
+                      const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total, long long pts_per_img,
+                      int n_sets, int S, int point, float box_scale, float* g_planes, float* g_dec, int fast, int skip, DetScratch* det, int sms,
+                      cudaStream_t st) {
   bwd::DetDecArgs a;
-  a.planes = planes; a.H = H; a.W = W; a.dec = dec; a.pts = pts; a.colours = colours; a.col_chunked = col_chunked; a.features = features; a.gsig = gsig; a.omega = omega;
+  a.planes = planes; a.H = H; a.W = W; a.n_sets = n_sets; a.dec = dec; a.pts = pts; a.colours = colours; a.col_chunked = col_chunked; a.features = features; a.gsig = gsig; a.omega = omega;
   a.g_rgb = g_rgb; a.total = total; a.pts_per_img = pts_per_img; a.S = S; a.box_scale = box_scale; a.g_planes = g_planes;
   a.g_dec = g_dec;
   a.g_acc = det ? det->acc : nullptr; a.dec_rows = det ? det->rows : nullptr; a.det_hdr = det ? det->hdr : nullptr;

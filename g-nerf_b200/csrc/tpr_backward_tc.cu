@@ -82,7 +82,7 @@ struct __align__(1024) Smem {
 };
 
 struct Args {
-  const float* planes; int H, W;        // packed [N,3,H,W,32]
+  const float* planes; int H, W;        // packed [P,3,H,W,32]: image n samples plane set n % n_sets
   const float* dec;                     // packed decoder
   const float* pts;                     // [T,3]
   const float* colours;                 // [T,32], or (col_chunked != 0) [rays, 8, S, 4] as tpr_render_train keeps them
@@ -100,6 +100,7 @@ struct Args {
   // kDet (deterministic mode): the plane gradient goes to g_acc in fixed point (scale 2^e from det_hdr), the decoder gradient
   // to this CTA's row of dec_rows; g_planes / g_dec only say whether each is wanted
   unsigned long long* g_acc; float* dec_rows; int* det_hdr;
+  int n_sets;                           // plane sets in planes / g_planes / g_acc
 };
 
 // ---- descriptors -------------------------------------------------------------------------------------------------
@@ -191,7 +192,8 @@ __global__ void scale_finish_kernel(const unsigned* __restrict__ acc, const floa
 // Deterministic mode: the fixed-point exponent e of the plane-gradient accumulator.  |GF_k| <= max|GA| . sum_j |W1t[k][j]|
 // and |GA| <= |GH| (softplus' <= 1) <= mg wc + ms wsig (the bound of scale_finish_kernel); a texel takes at most K samples'
 // contributions with tap weights of sum <= 1 per plane, so its sum is at most K . bound_GF and e = 62 - ceil(log2(K . bound_GF))
-// cannot overflow.  The bound scales exactly with the upstream gradient, so 2^k x the upstream gradient gives e - k and the
+// cannot overflow.  K = the samples that share one plane set: total / n_sets (with several images per set, F images add into
+// the same texels).  The bound scales exactly with the upstream gradient, so 2^k x the upstream gradient gives e - k and the
 // same integers.  A non-finite bound (inf upstream) or one whose e would leave the fp32 range marks the result NaN.
 __global__ void det_bound_kernel(const unsigned* __restrict__ acc, const float* __restrict__ dec, long long K, int* __restrict__ hdr) {
   __shared__ float col[64], row[32];
@@ -327,7 +329,10 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
           } else {                                 // not kept by the forward: gather again (VR/renderer.py:39-65)
             const float px = __fmul_rn(__ldg(a.pts + 3 * gs + 0), a.box_scale), py = __fmul_rn(__ldg(a.pts + 3 * gs + 1), a.box_scale),
                         pz = __fmul_rn(__ldg(a.pts + 3 * gs + 2), a.box_scale);
-            const int n = (int)n0 + (rem0 + sr >= a.pts_per_img ? 1 : 0);
+            int n = (int)n0 + (rem0 + sr >= a.pts_per_img ? 1 : 0);
+            // plane set n % n_sets, reduced only past the first n_sets images: a set index held across the tile (as the
+            // scatter does) costs these warps spill traffic at their 72-register budget
+            if (!kPoint && n >= a.n_sets) n = (int)((unsigned)n % (unsigned)a.n_sets);
             f[it] = gather_point(a.planes + (size_t)n * img_stride, a.H, a.W, px, py, pz, sub);
           }
         }
@@ -457,6 +462,7 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
       mbar_wait_parked(&s.gf_ready[b], (uint32_t)(i >> 1) & 1u);
       PROF(5);
       if (want_planes) {
+        const int set0 = kPoint ? (int)n0 : (int)n0 % a.n_sets;    // the plane set of the tile's first image (see LOAD)
 #pragma unroll
         for (int it = 0; it < 4; ++it) {
           const int sr = sw * 16 + it * 4 + grp;
@@ -467,7 +473,8 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
               float4 gf = *reinterpret_cast<const float4*>(s.gf[b] + row_chunk_off(sr, sub));
               gf = make_float4(gf.x * fx, gf.y * fx, gf.z * fx, gf.w * fx);
               if (!fixed_ok(gf)) a.det_hdr[1] = 1;
-              const int n = (int)n0 + (rem0 + sr >= a.pts_per_img ? 1 : 0);
+              int n = set0 + (rem0 + sr >= a.pts_per_img ? 1 : 0);
+              if (!kPoint && n == a.n_sets) n = 0;
               unsigned long long* img = a.g_acc + (size_t)n * img_stride + sub * 4;
               const float x = __fmul_rn(px[it], a.box_scale), y = __fmul_rn(py[it], a.box_scale), z = __fmul_rn(pz[it], a.box_scale);
 #pragma unroll
@@ -485,7 +492,8 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
               continue;
             }
             const float4 gf = *reinterpret_cast<const float4*>(s.gf[b] + row_chunk_off(sr, sub));
-            const int n = (int)n0 + (rem0 + sr >= a.pts_per_img ? 1 : 0);
+            int n = set0 + (rem0 + sr >= a.pts_per_img ? 1 : 0);
+            if (!kPoint && n == a.n_sets) n = 0;
             float* img = a.g_planes + (size_t)n * img_stride + sub * 4;
             const float x = __fmul_rn(px[it], a.box_scale), y = __fmul_rn(py[it], a.box_scale), z = __fmul_rn(pz[it], a.box_scale);
 #pragma unroll
@@ -738,12 +746,13 @@ __global__ void __launch_bounds__(kThreads, 1) decode_backward_tc_kernel(const A
 // Launch; returns cudaError_t (0 = ok) or -1 when the device cannot run it (the caller keeps the mma.sync kernel).
 // scale_buf: 4 floats of device scratch ([0..1] the power-of-two scale and its inverse, [2..3] the range accumulators).
 // point != 0: point queries (rows of colours / g_rgb per point, no omega, S unused; g_rgb may be NULL).
+// n_sets: planes / g_planes hold n_sets plane sets; image n (of total / pts_per_img) reads and scatters to set n % n_sets.
 // det != NULL: the deterministic mode (tpr_device.cuh: DetScratch); the launch sets det->n_rows and zeroes those rows, the
 // caller zeroes det->acc and converts both afterwards (launch_det_finish).
 int launch_bwd_decode_tc(const float* planes, int H, int W, const float* dec, const float* pts, const float* colours, int col_chunked,
                          const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total,
-                         long long pts_per_img, int S, int point, float box_scale, float* g_planes, float* g_dec, float* scale_buf,
-                         DetScratch* det, int sms, int smem_optin, cudaStream_t st) {
+                         long long pts_per_img, int n_sets, int S, int point, float box_scale, float* g_planes, float* g_dec,
+                         float* scale_buf, DetScratch* det, int sms, int smem_optin, cudaStream_t st) {
   using namespace bwdtc;
   const size_t smem = sizeof(Smem) + 1024 + (det ? kLoadWarps * 33 * sizeof(float) : 0);
   if ((int)smem > smem_optin) return -1;
@@ -752,9 +761,9 @@ int launch_bwd_decode_tc(const float* planes, int H, int W, const float* dec, co
   const long long n_rgb = point ? (g_rgb ? total * 32 : 0) : (total / S) * 32;
   scale_kernel<<<sms * 4, 256, 0, st>>>(g_rgb, n_rgb, gsig, total, dec, reinterpret_cast<unsigned*>(scale_buf + 2));
   scale_finish_kernel<<<1, 64, 0, st>>>(reinterpret_cast<const unsigned*>(scale_buf + 2), dec, scale_buf);
-  if (det) det_bound_kernel<<<1, 64, 0, st>>>(reinterpret_cast<const unsigned*>(scale_buf + 2), dec, pts_per_img, det->hdr);
+  if (det) det_bound_kernel<<<1, 64, 0, st>>>(reinterpret_cast<const unsigned*>(scale_buf + 2), dec, total / n_sets, det->hdr);
   Args a;
-  a.planes = planes; a.H = H; a.W = W; a.dec = dec; a.pts = pts; a.colours = colours; a.col_chunked = col_chunked; a.features = features; a.gsig = gsig;
+  a.planes = planes; a.H = H; a.W = W; a.n_sets = n_sets; a.dec = dec; a.pts = pts; a.colours = colours; a.col_chunked = col_chunked; a.features = features; a.gsig = gsig;
   a.omega = omega; a.g_rgb = g_rgb; a.total = total; a.pts_per_img = pts_per_img; a.S = S; a.box_scale = box_scale;
   a.g_planes = g_planes; a.g_dec = g_dec; a.scale = scale_buf; a.prof = nullptr;
   a.g_acc = det ? det->acc : nullptr; a.dec_rows = det ? det->rows : nullptr; a.det_hdr = det ? det->hdr : nullptr;
@@ -799,14 +808,14 @@ int launch_bwd_decode_tc(const float* planes, int H, int W, const float* dec, co
 
 // Deterministic mode ahead of the mma.sync kernel: the upstream gradient's range and the fixed-point exponent into det->hdr
 // (what launch_bwd_decode_tc computes on its way).  Arguments as there.
-int launch_det_bound(const float* dec, const float* gsig, const float* g_rgb, long long total, long long pts_per_img, int S, int point,
+int launch_det_bound(const float* dec, const float* gsig, const float* g_rgb, long long total, int n_sets, int S, int point,
                      float* scale_buf, DetScratch* det, int sms, cudaStream_t st) {
   using namespace bwdtc;
   cudaError_t e = cudaMemsetAsync(scale_buf + 2, 0, 2 * sizeof(float), st);
   if (e != cudaSuccess) return (int)e;
   const long long n_rgb = point ? (g_rgb ? total * 32 : 0) : (total / S) * 32;
   scale_kernel<<<sms * 4, 256, 0, st>>>(g_rgb, n_rgb, gsig, total, dec, reinterpret_cast<unsigned*>(scale_buf + 2));
-  det_bound_kernel<<<1, 64, 0, st>>>(reinterpret_cast<const unsigned*>(scale_buf + 2), dec, pts_per_img, det->hdr);
+  det_bound_kernel<<<1, 64, 0, st>>>(reinterpret_cast<const unsigned*>(scale_buf + 2), dec, total / n_sets, det->hdr);
   return (int)cudaGetLastError();
 }
 

@@ -48,6 +48,7 @@ constexpr uint32_t kRmSlotBase = kStages * kRmStageCols;
 
 struct RmArgs {
   const float* planes; int H, W;
+  long long plane_sets;            // image n reads plane set n % plane_sets
   const float* dec; const float* xyz;
   long long n_pts, tiles_per_img, n_tiles;
   float box_scale;
@@ -152,7 +153,7 @@ run_model_ws_kernel(const RmArgs a) {
       mbar_wait_parked(&bars.a1_free[b], ph ^ 1u);          // passes immediately the first time round
 #pragma unroll 1
       for (int ps = 0; ps < Roles<RGB>::passes; ++ps)
-        gather_tile_points<MODE>(a, tl.a1[b][0], a.planes + (size_t)n * img_stride,
+        gather_tile_points<MODE>(a, tl.a1[b][0], a.planes + (size_t)(n % a.plane_sets) * img_stride,
                                  a.xyz + (size_t)(n * a.n_pts + p0) * 3, nvalid, tw, (wt * Roles<RGB>::passes + ps) * 8, lane);
       fence_proxy_async_smem();
       __syncwarp();
@@ -256,11 +257,11 @@ static size_t smem_bytes() { return 1024 + sizeof(Tiles<MODE>) + sizeof(Tap2) * 
 }  // namespace wsrm
 
 // Launch; returns cudaError_t (0 = ok) or -1 if the shape does not fit (the caller uses the FFMA kernel).
-int launch_run_model_ws(const float* planes, long long n_img, int H, int W, const float* dec, const float* xyz, long long n_pts,
-                        float box_scale, float* rgb, float* sigma, int mode, int sms, int smem_optin, cudaStream_t st) {
+int launch_run_model_ws(const float* planes, long long n_img, long long plane_sets, int H, int W, const float* dec, const float* xyz,
+                        long long n_pts, float box_scale, float* rgb, float* sigma, int mode, int sms, int smem_optin, cudaStream_t st) {
   using namespace wsrm;
   RmArgs a;
-  a.planes = planes; a.H = H; a.W = W; a.dec = dec; a.xyz = xyz; a.n_pts = n_pts;
+  a.planes = planes; a.H = H; a.W = W; a.plane_sets = plane_sets; a.dec = dec; a.xyz = xyz; a.n_pts = n_pts;
   a.tiles_per_img = (n_pts + ws::kRows - 1) / ws::kRows;
   a.n_tiles = a.tiles_per_img * n_img;
   a.box_scale = box_scale; a.rgb = rgb; a.sigma = sigma;

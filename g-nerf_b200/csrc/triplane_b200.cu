@@ -23,26 +23,26 @@ int ws_rays_per_group(int Dc, int Df, int mode);
 bool ws_keeps_samples(int Dc, int Df);
 int launch_render_ws(RenderArgs a, int mode, int sms, int smem_optin, long long n_img, long long n_rays, cudaStream_t st);
 // tpr_run_model_ws.cu
-int launch_run_model_ws(const float* planes, long long n_img, int H, int W, const float* dec, const float* xyz, long long n_pts,
-                        float box_scale, float* rgb, float* sigma, int mode, int sms, int smem_optin, cudaStream_t st);
+int launch_run_model_ws(const float* planes, long long n_img, long long plane_sets, int H, int W, const float* dec, const float* xyz,
+                        long long n_pts, float box_scale, float* rgb, float* sigma, int mode, int sms, int smem_optin, cudaStream_t st);
 
 // tpr_backward.cu
 int launch_bwd_points(const float* origins, const float* dirs, const float* dc, const float* df, int Dc, int Df,
                       long long n_rays_total, float* pts, int sms, cudaStream_t st);
 int launch_bwd_march(const float* dc, const float* df, int Dc, int Df, const float* sigma, const float* colours, int col_chunked,
-                     const float* g_rgb, const float* g_depth, const float* g_wsum, const float* range, int white_back,
-                     long long n_rays_total, float* gsig, float* omega, int sms, cudaStream_t st);
+                     const float* g_rgb, const float* g_depth, const float* g_wsum, const float* range, long long group_rays,
+                     int white_back, long long n_rays_total, float* gsig, float* omega, int sms, cudaStream_t st);
 int launch_bwd_decode(const float* planes, int H, int W, const float* dec, const float* pts, const float* colours, int col_chunked,
-                      const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total, long long pts_per_img, int S,
-                      int point, float box_scale, float* g_planes, float* g_dec, int fast, int skip, DetScratch* det, int sms,
+                      const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total, long long pts_per_img,
+                      int n_sets, int S, int point, float box_scale, float* g_planes, float* g_dec, int fast, int skip, DetScratch* det, int sms,
                       cudaStream_t st);
 int launch_det_finish(const DetScratch* det, long long n_plane_floats, float* g_planes, float* g_dec, int sms, cudaStream_t st);
 // tpr_backward_tc.cu: the decoder backward on tcgen05 (returns -1 if it cannot run here)
 int launch_bwd_decode_tc(const float* planes, int H, int W, const float* dec, const float* pts, const float* colours, int col_chunked,
                          const float* features, const float* gsig, const float* omega, const float* g_rgb, long long total,
-                         long long pts_per_img, int S, int point, float box_scale, float* g_planes, float* g_dec, float* scale_buf,
-                         DetScratch* det, int sms, int smem_optin, cudaStream_t st);
-int launch_det_bound(const float* dec, const float* gsig, const float* g_rgb, long long total, long long pts_per_img, int S, int point,
+                         long long pts_per_img, int n_sets, int S, int point, float box_scale, float* g_planes, float* g_dec,
+                         float* scale_buf, DetScratch* det, int sms, int smem_optin, cudaStream_t st);
+int launch_det_bound(const float* dec, const float* gsig, const float* g_rgb, long long total, int n_sets, int S, int point,
                      float* scale_buf, DetScratch* det, int sms, cudaStream_t st);
 int launch_unpack_decoder_grad(const float* gd, float g_w1, float g_b1, float g_w2, float g_b2, float* w1, float* b1, float* w2,
                                float* b2, cudaStream_t st);
@@ -204,7 +204,7 @@ template <bool kFromFeatures>
 __global__ void __launch_bounds__(kRmThreads) run_model_kernel(
     const float* __restrict__ planes, int H, int W, const float* __restrict__ dec,
     const float* __restrict__ in /* xyz [N,P,3] or features [N,3,P,32] */, long long n_img, long long n_pts,
-    float box_scale, float* __restrict__ rgb, float* __restrict__ sigma) {
+    float box_scale, float* __restrict__ rgb, float* __restrict__ sigma, long long plane_sets /* image n reads set n % plane_sets */) {
   extern __shared__ __align__(16) float smem[];
   float* wsm = smem;
   float* rows = smem + kDecFloats + (threadIdx.x >> 5) * 32 * kC;
@@ -228,7 +228,7 @@ __global__ void __launch_bounds__(kRmThreads) run_model_kernel(
         py = __fmul_rn(in[g * 3 + 1], box_scale);
         pz = __fmul_rn(in[g * 3 + 2], box_scale);
       }
-      gather_chunk(planes + n * img_stride, H, W, px, py, pz, lane, valid, rows, lane);
+      gather_chunk(planes + (size_t)(n % plane_sets) * img_stride, H, W, px, py, pz, lane, valid, rows, lane);
     } else {
       // features [N,3,P,32]: sum the three planes' rows, eight lanes per sample
       const int grp = lane >> 3, sub = lane & 7;
@@ -716,7 +716,9 @@ int tpr_sample_stratified(const float* jitter, int64_t n_rays, const float* ray_
   return 0;
 }
 
-static int launch_run_model(bool from_features, const float* planes, int64_t n_img, int32_t H, int32_t W,
+// plane_sets: image n reads plane set n % plane_sets (tpr_run_model: plane_sets = n_img; the render backward re-evaluates
+// frame-batched samples with the forward's plane_sets)
+static int launch_run_model(bool from_features, const float* planes, int64_t n_img, int64_t plane_sets, int32_t H, int32_t W,
                             const float* dec, const float* in, int64_t n_pts, double box_warp, float* rgb, float* sigma,
                             int32_t flags, void* stream) {
   if (!dec || !in || !sigma) return fail(TPR_E_NULL, "run_model: NULL pointer");
@@ -734,7 +736,7 @@ static int launch_run_model(bool from_features, const float* planes, int64_t n_i
   // fp32 FFMA kernel below, whose 32-point chunks spread over the SMs at any size.
   if (!from_features && flags != TPR_MLP_FFMA && (long long)n_img * n_pts >= env_int("TPR_RM_WS_MIN_POINTS", 1 << 16) &&
       !env_int("TPR_FORCE_FFMA", 0)) {
-    int rc = launch_run_model_ws(planes, n_img, H, W, dec, in, n_pts, box_scale, rgb, sigma, tc_mode(flags), di.sms,
+    int rc = launch_run_model_ws(planes, n_img, plane_sets, H, W, dec, in, n_pts, box_scale, rgb, sigma, tc_mode(flags), di.sms,
                                  di.smem_optin, (cudaStream_t)stream);
     if (rc > 0) return cuda_fail((cudaError_t)rc, "run_model_ws_kernel");
     if (rc == 0) return 0;
@@ -751,23 +753,24 @@ static int launch_run_model(bool from_features, const float* planes, int64_t n_i
   const long long total = (long long)n_img * n_pts;
   const int grid = grid_for(total, kRmThreads, di.sms, env_int("TPR_RM_WAVES", 3));
   if (from_features)
-    run_model_kernel<true><<<grid, kRmThreads, smem, (cudaStream_t)stream>>>(nullptr, 0, 0, dec, in, n_img, n_pts, 0.f, rgb, sigma);
+    run_model_kernel<true><<<grid, kRmThreads, smem, (cudaStream_t)stream>>>(nullptr, 0, 0, dec, in, n_img, n_pts, 0.f, rgb, sigma, 1);
   else
-    run_model_kernel<false><<<grid, kRmThreads, smem, (cudaStream_t)stream>>>(planes, H, W, dec, in, n_img, n_pts, box_scale, rgb, sigma);
+    run_model_kernel<false><<<grid, kRmThreads, smem, (cudaStream_t)stream>>>(planes, H, W, dec, in, n_img, n_pts, box_scale, rgb, sigma,
+                                                                          plane_sets);
   TPR_CHECK_LAUNCH("run_model_kernel");
   return 0;
 }
 
 int tpr_run_model(const float* planes_packed, int64_t n_img, int32_t height, int32_t width, const float* decoder_packed,
                   const float* xyz, int64_t n_pts, double box_warp, float* rgb, float* sigma, int32_t flags, void* stream) {
-  return launch_run_model(false, planes_packed, n_img, height, width, decoder_packed, xyz, n_pts, box_warp, rgb, sigma,
+  return launch_run_model(false, planes_packed, n_img, n_img, height, width, decoder_packed, xyz, n_pts, box_warp, rgb, sigma,
                           flags, stream);
 }
 
 int tpr_decode(const float* features, int64_t n_img, int64_t n_pts, const float* decoder_packed, float* rgb, float* sigma,
                int32_t flags, void* stream) {
   if (!rgb) return fail(TPR_E_NULL, "tpr_decode: NULL rgb");
-  return launch_run_model(true, nullptr, n_img, 0, 0, decoder_packed, features, n_pts, 1.0, rgb, sigma, flags, stream);
+  return launch_run_model(true, nullptr, n_img, 1, 0, 0, decoder_packed, features, n_pts, 1.0, rgb, sigma, flags, stream);
 }
 
 // [0..8) call-wide depth range, [64..192) phase counters, from byte 256 one (min, max) pair per depth-clamp slot
@@ -1258,7 +1261,8 @@ size_t tpr_render_backward_scratch_bytes(int64_t n_img, int64_t n_rays, int32_t 
   return align256(T * 12) + align256(T * 128) + 3 * align256(T * 4) + 256;
 }
 
-// TPR_BWD_DETERMINISTIC: [256 B: DetScratch::hdr][kDetMaxRows decoder rows][int64 accumulator [N,3,H,W,32]]
+// TPR_BWD_DETERMINISTIC: [256 B: DetScratch::hdr][kDetMaxRows decoder rows][int64 accumulator [P,3,H,W,32]]; P = the plane
+// sets (tpr_render_backward with plane_sets > 0), else the images
 size_t tpr_backward_deterministic_scratch_bytes(int64_t n_img, int32_t height, int32_t width) {
   if (n_img <= 0 || height <= 0 || width <= 0) return 0;
   return 256 + align256((size_t)kDetMaxRows * kDecFloats * sizeof(float)) +
@@ -1276,13 +1280,14 @@ static DetScratch det_scratch(void* scratch, size_t base) {
 
 // The decoder backward of both entry points: tcgen05 + TMEM, warp-specialised (tpr_backward_tc.cu) first; the mma.sync kernel
 // when it refuses (fewer than 128 samples per image, too little shared memory) or with TPR_BWD_IMPL=hmma (A/B runs).  The outputs
-// are zeroed here.  det != NULL: the deterministic mode, its outputs converted after the kernel.
-static int decoder_backward(const float* planes_packed, int64_t n_img, int32_t height, int32_t width, const float* dec, const float* pts,
+// are zeroed here.  det != NULL: the deterministic mode, its outputs converted after the kernel.  n_sets: the plane sets in
+// planes_packed / g_planes_packed (image n = sample / pts_per_img reads and scatters to set n % n_sets).
+static int decoder_backward(const float* planes_packed, int n_sets, int32_t height, int32_t width, const float* dec, const float* pts,
                             const float* colours, int col_chunked, const float* features, const float* gsig, const float* omega,
                             const float* g_rgb, long long total, long long pts_per_img, int S, int point, float box_scale, int fast,
                             float* g_planes_packed, float* g_decoder_packed, float* scale_buf, void* scratch, DetScratch* det,
                             const DeviceInfo& di, cudaStream_t st) {
-  const size_t plane_floats = (size_t)n_img * 3 * height * width * kC;
+  const size_t plane_floats = (size_t)n_sets * 3 * height * width * kC;
   cudaError_t e = cudaSuccess;
   if (g_planes_packed) e = det ? cudaMemsetAsync(det->acc, 0, plane_floats * sizeof(long long), st)
                                : cudaMemsetAsync(g_planes_packed, 0, plane_floats * sizeof(float), st);
@@ -1292,18 +1297,18 @@ static int decoder_backward(const float* planes_packed, int64_t n_img, int32_t h
   int rc = -1;
   if (!(impl && strcmp(impl, "hmma") == 0)) {
     rc = launch_bwd_decode_tc(planes_packed, height, width, dec, pts, colours, col_chunked, features, gsig, omega, g_rgb, total,
-                              pts_per_img, S, point, box_scale, g_planes_packed, g_decoder_packed, scale_buf, det, di.sms,
+                              pts_per_img, n_sets, S, point, box_scale, g_planes_packed, g_decoder_packed, scale_buf, det, di.sms,
                               di.smem_optin, st);
     if (rc > 0) return cuda_fail((cudaError_t)rc, "decode_backward_tc_kernel");
   }
   if (rc != 0) {
     if (det) {
-      rc = launch_det_bound(dec, gsig, g_rgb, total, pts_per_img, S, point, scale_buf, det, di.sms, st);
+      rc = launch_det_bound(dec, gsig, g_rgb, total, n_sets, S, point, scale_buf, det, di.sms, st);
       if (rc != 0) return cuda_fail((cudaError_t)rc, "det_bound_kernel");
     }
     float* g_dec_out = g_decoder_packed ? g_decoder_packed : reinterpret_cast<float*>(scratch);      // (never written when skipped)
     rc = launch_bwd_decode(planes_packed, height, width, dec, pts, colours, col_chunked, features, gsig, omega, g_rgb, total,
-                           pts_per_img, S, point, box_scale, g_planes_packed, g_dec_out, fast,
+                           pts_per_img, n_sets, S, point, box_scale, g_planes_packed, g_dec_out, fast,
                            (g_planes_packed ? 0 : 1) | (g_decoder_packed ? 0 : 2), det, di.sms, st);
     if (rc != 0) return cuda_fail((cudaError_t)rc, "decode_backward_kernel");
   }
@@ -1324,7 +1329,7 @@ int tpr_march_backward(const float* depths_coarse, const float* depths_fine, int
   if (n_rays_total <= 0 || dc < 2 || df < 0 || dc + df > TPR_MAX_SAMPLES) return fail(TPR_E_SHAPE, "tpr_march_backward: bad shape");
   DeviceInfo di = device_info();
   if (!di.ok) return fail(TPR_E_DEVICE, "tpr_march_backward: no CUDA device");
-  const int rc = launch_bwd_march(depths_coarse, depths_fine, dc, df, sigma, colours, 0, g_rgb, g_depth, g_weight_sum, depth_range,
+  const int rc = launch_bwd_march(depths_coarse, depths_fine, dc, df, sigma, colours, 0, g_rgb, g_depth, g_weight_sum, depth_range, 0,
                                   white_back, n_rays_total, g_sigma, omega, di.sms, (cudaStream_t)stream);
   if (rc != 0) return cuda_fail((cudaError_t)rc, "march_backward_kernel");
   return 0;
@@ -1345,15 +1350,20 @@ int tpr_render_backward(const float* planes_packed, int64_t n_img, int32_t heigh
   if (n_img <= 0 || n_rays <= 0 || height <= 0 || width <= 0 || Dc < 2 || Df < 0 || S > TPR_MAX_SAMPLES)
     return fail(TPR_E_SHAPE, "tpr_render_backward: bad shape");
   if ((long long)3 * height * width * kC >= (1ll << 32)) return fail(TPR_E_SHAPE, "tpr_render_backward: planes too large");
-  if (opt->plane_sets != 0 && opt->plane_sets != n_img) return fail(TPR_E_OPTION, "tpr_render_backward: one plane set per image only");
-  if (opt->depth_clamp_group != 0) return fail(TPR_E_OPTION, "tpr_render_backward: depth_clamp_group is not supported");
+  if (n_img >= (1ll << 31)) return fail(TPR_E_SHAPE, "tpr_render_backward: too many images");
+  if (opt->plane_sets < 0 || (opt->plane_sets > 0 && n_img % opt->plane_sets != 0))
+    return fail(TPR_E_SHAPE, "tpr_render_backward: n_img must be a multiple of plane_sets");
+  if (opt->depth_clamp_group < 0) return fail(TPR_E_OPTION, "tpr_render_backward: depth_clamp_group < 0");
+  if (opt->depth_clamp_group > 0 && n_img * n_rays >= (1ll << 32))
+    return fail(TPR_E_SHAPE, "tpr_render_backward: depth_clamp_group needs fewer than 2^32 rays");
+  const int P = opt->plane_sets > 0 ? opt->plane_sets : (int)n_img;
   if (!(opt->box_warp > 0)) return fail(TPR_E_OPTION, "tpr_render_backward: box_warp must be > 0");
   const bool det = (opt->flags & TPR_BWD_DETERMINISTIC) != 0;
   const int32_t mlp = opt->flags & ~TPR_BWD_DETERMINISTIC;
   if (mlp != TPR_MLP_FP32 && mlp != TPR_MLP_BF16 && mlp != TPR_MLP_FFMA)
     return fail(TPR_E_OPTION, "tpr_render_backward: unknown flag");
   const size_t base_bytes = tpr_render_backward_scratch_bytes(n_img, n_rays, S);
-  if (scratch_bytes < base_bytes + (det ? tpr_backward_deterministic_scratch_bytes(n_img, height, width) : 0))
+  if (scratch_bytes < base_bytes + (det ? tpr_backward_deterministic_scratch_bytes(P, height, width) : 0))
     return fail(TPR_E_SCRATCH, "tpr_render_backward: scratch too small");
   DeviceInfo di = device_info();
   if (!di.ok) return fail(TPR_E_DEVICE, "tpr_render_backward: no CUDA device");
@@ -1374,16 +1384,18 @@ int tpr_render_backward(const float* planes_packed, int64_t n_img, int32_t heigh
   if (!col_in) {
     // not kept by the forward (tpr_render_train): colours and densities of every sample through the forward's point query
     // (VR/renderer.py:142-148)
-    rc = tpr_run_model(planes_packed, n_img, height, width, decoder_packed, pts, (int64_t)n_rays * S, opt->box_warp, colours, sigma,
-                       mlp, stream);
+    rc = launch_run_model(false, planes_packed, n_img, P, height, width, decoder_packed, pts, (int64_t)n_rays * S, opt->box_warp,
+                          colours, sigma, mlp, stream);
     if (rc != 0) return rc;
     col_in = colours; sig_in = sigma;
   }
+  // a group of k >= n_img cameras is the whole call: min(k, n_img) rays_per_img keeps the group size <= the rays (< 2^32)
+  const long long group_rays = opt->depth_clamp_group > 0 ? (opt->depth_clamp_group < n_img ? (long long)opt->depth_clamp_group : (long long)n_img) * n_rays : 0;
   rc = launch_bwd_march(depths_coarse, depths_fine, Dc, Df, sig_in, col_in, col_chunked, g_rgb, g_depth, g_weight_sum, depth_range,
-                        opt->white_back, rays, gsig, omega, di.sms, st);
+                        group_rays, opt->white_back, rays, gsig, omega, di.sms, st);
   if (rc != 0) return cuda_fail((cudaError_t)rc, "march_backward_kernel");
   DetScratch ds = det_scratch(scratch, base_bytes);
-  return decoder_backward(planes_packed, n_img, height, width, decoder_packed, pts, col_in, col_chunked, sample_features, gsig, omega,
+  return decoder_backward(planes_packed, P, height, width, decoder_packed, pts, col_in, col_chunked, sample_features, gsig, omega,
                           g_rgb, (long long)T, (long long)n_rays * S, S, 0, (float)(2.0 / opt->box_warp), mlp == TPR_MLP_BF16,
                           g_planes_packed, g_decoder_packed, scale_buf, scratch, det ? &ds : nullptr, di, st);
 }
@@ -1429,7 +1441,7 @@ int tpr_run_model_backward(const float* planes_packed, int64_t n_img, int32_t he
   const float* gsig = g_sigma ? g_sigma : zero_gsig;
   const float box_scale = (float)(2.0 / box_warp);      // python float (VR/renderer.py:61)
   DetScratch ds = det_scratch(scratch, base_bytes);
-  return decoder_backward(planes_packed, n_img, height, width, decoder_packed, xyz, rgb, 0, nullptr, gsig, nullptr, g_rgb, T, n_pts, 1, 1,
+  return decoder_backward(planes_packed, (int)n_img, height, width, decoder_packed, xyz, rgb, 0, nullptr, gsig, nullptr, g_rgb, T, n_pts, 1, 1,
                           box_scale, flags == TPR_MLP_BF16, g_planes_packed, g_decoder_packed, scale_buf, scratch, det ? &ds : nullptr,
                           di, st);
 }

@@ -49,10 +49,19 @@ def render_frames(renderer, planes, decoder, cam2world, intrinsics, resolution, 
     Returns the neural-rendered images exactly as TriPlaneGenerator.synthesis shapes them (training/triplane.py:81-82):
     ``feature_image`` [F,P,32,res,res], ``depth_image`` [F,P,1,res,res], ``weights_image`` [F,P,1,res,res]; the feature
     image is written channels-first by the kernel (no permute + contiguous pass).
+
+    Under autograd (``planes`` or the decoder's parameters require grad) the three images are attached to them: each chunk
+    of ``frames_per_call`` frames is one differentiable forward over the planes tensor (one autograd node; the backward
+    scatters every frame's gradient into the P plane sets at once), and the images are views of its outputs (one chunk) or
+    their concatenation.  Same noise draws and outputs as without autograd.
     """
-    pp = renderer._packed(planes) if hasattr(renderer, '_packed') else _r.pack_planes(planes)
-    P = pp.n_img
-    dev = pp.device
+    grad = torch.is_grad_enabled() and _r._wants_grad(planes, decoder)
+    if grad and isinstance(planes, torch.Tensor):
+        # the forward repacks the tensor itself (render_with_grad); PackedPlanes keep the inference path, which refuses them
+        src, P, dev = planes, planes.shape[0], planes.device
+    else:
+        src = renderer._packed(planes) if hasattr(renderer, '_packed') else _r.pack_planes(planes)
+        P, dev = src.n_img, src.device
     cam2world = torch.as_tensor(cam2world, dtype=torch.float32, device=dev)
     intrinsics = torch.as_tensor(intrinsics, dtype=torch.float32, device=dev)
     if cam2world.dim() == 3:
@@ -71,9 +80,11 @@ def render_frames(renderer, planes, decoder, cam2world, intrinsics, resolution, 
     m = res * res
     dc, df = int(rendering_options['depth_resolution']), int(rendering_options['depth_resolution_importance'])
     opts = dict(rendering_options, output_layout='channels_first', depth_clamp_group=P)
-    feat = torch.empty((F, P, 32, res, res), device=dev, dtype=torch.float32)
-    depth = torch.empty((F, P, 1, res, res), device=dev, dtype=torch.float32)
-    wsum = torch.empty((F, P, 1, res, res), device=dev, dtype=torch.float32)
+    if not grad:
+        feat = torch.empty((F, P, 32, res, res), device=dev, dtype=torch.float32)
+        depth = torch.empty((F, P, 1, res, res), device=dev, dtype=torch.float32)
+        wsum = torch.empty((F, P, 1, res, res), device=dev, dtype=torch.float32)
+    chunks = []
     step = F if not frames_per_call else max(1, int(frames_per_call))
     with torch.cuda.device(dev):
         if noise is None:
@@ -83,11 +94,20 @@ def render_frames(renderer, planes, decoder, cam2world, intrinsics, resolution, 
             f1 = min(F, f0 + step)
             n = (f1 - f0) * P
             o, d = sampler(cam2world[f0:f1].reshape(n, 4, 4).contiguous(), intrinsics[f0:f1].reshape(n, 3, 3).contiguous(), res)
-            out = (feat[f0:f1].view(n, 32, m).permute(0, 2, 1), depth[f0:f1].view(n, m, 1), wsum[f0:f1].view(n, m, 1))
             nz = (jitter[f0 * P:f1 * P], u[f0 * P * m:f1 * P * m] if u is not None else None)
             if len(noise) == 4:
                 nz = nz + (noise[2][f0 * P:f1 * P], noise[3][f0 * P:f1 * P] if noise[3] is not None else None)
-            _r.ImportanceRenderer.forward(renderer, pp, decoder, o, d, opts, noise=nz, out=out)
+            if grad:
+                # rgb is the [n,M,32] view of [n,32,M] memory (channels_first): the [f,P,32,res,res] image is a free view
+                rgb, dep, ws = _r.ImportanceRenderer.forward(renderer, src, decoder, o, d, opts, noise=nz)
+                f = f1 - f0
+                chunks.append((rgb.permute(0, 2, 1).view(f, P, 32, res, res), dep.view(f, P, 1, res, res),
+                               ws.view(f, P, 1, res, res)))
+                continue
+            out = (feat[f0:f1].view(n, 32, m).permute(0, 2, 1), depth[f0:f1].view(n, m, 1), wsum[f0:f1].view(n, m, 1))
+            _r.ImportanceRenderer.forward(renderer, src, decoder, o, d, opts, noise=nz, out=out)
+    if grad:
+        feat, depth, wsum = chunks[0] if len(chunks) == 1 else (torch.cat(t, 0) for t in zip(*chunks))
     return {'feature_image': feat, 'depth_image': depth, 'weights_image': wsum}
 
 

@@ -8,6 +8,14 @@ runs the march, the decoder and the bilinear gather backwards.  Saved between th
 decoder, the rays, the S sample depths per ray, the depth range and -- written by the forward kernel's composite on its
 way -- the 32 colours and sigma of every sample (132 B per sample; eager autograd keeps ~800 B per sample).
 
+Frame-batched renders (F*P cameras over P plane sets, camera n sampling set n % P: ``TprOptions.plane_sets``, what
+frames.render_frames passes) differentiate as one call: the backward reads and scatters set n % P, so every plane set
+receives the sum of its F cameras' gradients in one [P,3,H,W,32] buffer.  With ``depth_clamp_group`` = k the depth of a
+camera was clamped to the range of its own group of k cameras; the forward keeps those ranges only in its scratch, so they
+are re-derived here as the min and max of each group's coarse and importance depths -- the values the forward reduced.
+``output_layout='channels_first'``: the rgb returned is the [N,M,32] view of [N,32,M] memory; its upstream gradient is
+copied once into the [N,M,32] rows the kernels read.
+
 The graph is the reference's: importance depths are constants (VR/renderer.py:198,210: no_grad + detach), so is the
 jitter; ray origins / directions are not differentiated (they raise if they require grad).
 
@@ -39,8 +47,9 @@ class _Render(torch.autograd.Function):
         s_col, s_sig, s_feat = aux['saved'] if ctx.has_saved else (None, None, None)
         ctx.has_feat = s_feat is not None
         empty = torch.empty(0, device=rgb.device)
+        rng = _group_ranges(aux['coarse'], aux['fine'], ctx.shape[0], aux['options'].depth_clamp_group, aux['range'])
         ctx.save_for_backward(aux['packed'].data, aux['dec'], origins.contiguous(), dirs.contiguous(), aux['coarse'], fine,
-                              aux['range'], s_col if ctx.has_saved else empty, s_sig if ctx.has_saved else empty,
+                              rng, s_col if ctx.has_saved else empty, s_sig if ctx.has_saved else empty,
                               s_feat if ctx.has_feat else empty)
         return rgb, depth, wsum
 
@@ -54,6 +63,7 @@ class _Render(torch.autograd.Function):
         L = _lib.lib()
         p, st = _r._ptr, _r._stream
         zeros = lambda shape: torch.zeros(shape, device=dev, dtype=torch.float32)
+        # (channels-first output: g_rgb usually arrives with the output's [N,32,M] strides; contiguous() is then one copy)
         g_rgb = g_rgb.contiguous().float() if g_rgb is not None else zeros((n, m, 32))
         g_depth = g_depth.contiguous().float() if g_depth is not None else zeros((n, m, 1))
         g_wsum = g_wsum.contiguous().float() if g_wsum is not None else zeros((n, m, 1))
@@ -63,11 +73,11 @@ class _Render(torch.autograd.Function):
             g_planes = torch.empty_like(packed) if want_planes else None
             g_dec = torch.empty_like(dec) if want_dec else None
             nbytes = L.tpr_render_backward_scratch_bytes(n, m, o.depth_resolution + o.depth_resolution_importance)
-            o2 = _lib.TprOptions.from_buffer_copy(o)
-            o2.plane_sets, o2.depth_clamp_group = 0, 0
+            o2 = _lib.TprOptions.from_buffer_copy(o)           # plane_sets / depth_clamp_group as the forward had them
             if torch.are_deterministic_algorithms_enabled():
                 o2.flags |= _lib.BWD_DETERMINISTIC
-                nbytes += L.tpr_backward_deterministic_scratch_bytes(n, pp.height, pp.width)
+                # the fixed-point accumulator holds the P plane sets, not the N cameras
+                nbytes += L.tpr_backward_deterministic_scratch_bytes(pp.n_img, pp.height, pp.width)
             scratch = torch.empty(nbytes, device=dev, dtype=torch.uint8)
             _lib.check(L.tpr_render_backward(p(packed), n, pp.height, pp.width, p(dec), p(origins), p(dirs), m, p(coarse),
                                              p(fine) if ctx.has_fine else None, p(rng), ctypes.byref(o2), p(g_rgb), p(g_depth),
@@ -79,6 +89,24 @@ class _Render(torch.autograd.Function):
         return (None, None, None, None, g_nchw,
                 g_w1 if need[5] else None, g_b1 if need[6] else None, g_w2 if need[7] else None, g_b2 if need[8] else None,
                 None, None)
+
+
+def _group_ranges(coarse, fine, n, k, rng):
+    """The depth-clamp ranges the forward used: ``rng`` [2] (its call-wide range) for k == 0, else [2*ceil(n/k)] = the (min,
+    max) of the coarse and importance depths of cameras [j k, j k + k) -- the reduction the forward made over the same
+    values, so the result is bit-equal to the ranges it clamped with."""
+    if k <= 0:
+        return rng
+    c = coarse.reshape(n, -1)
+    lo, hi = c.amin(1), c.amax(1)
+    if fine is not None and fine.numel():                           # (min / max commute: no concatenated copy)
+        f = fine.reshape(n, -1)
+        lo, hi = torch.minimum(lo, f.amin(1)), torch.maximum(hi, f.amax(1))
+    g = -(-n // k)
+    pad = g * k - n                                                  # a shorter last group
+    lo = torch.nn.functional.pad(lo, (0, pad), value=float('inf')).view(g, k).amin(1)
+    hi = torch.nn.functional.pad(hi, (0, pad), value=float('-inf')).view(g, k).amax(1)
+    return torch.stack([lo, hi], 1).reshape(-1).contiguous()
 
 
 def _unpack_grads(g_planes, g_dec, gains, pp, dev):
@@ -103,16 +131,13 @@ def _unpack_grads(g_planes, g_dec, gains, pp, dev):
 
 def render_with_grad(renderer, planes, decoder, ray_origins, ray_directions, options, noise=None):
     """ImportanceRenderer.forward with autograd: returns (rgb, depth, weight_sum) attached to ``planes`` and to the
-    decoder's parameters."""
+    decoder's parameters.  Takes every forward option: frame batching (N = F*P cameras over P plane sets),
+    ``depth_clamp_group`` and ``output_layout='channels_first'`` included."""
     if isinstance(planes, _r.PackedPlanes):
         raise NotImplementedError('autograd needs the planes tensor itself ([N,3,32,H,W]), not PackedPlanes')
     for t, name in ((ray_origins, 'ray_origins'), (ray_directions, 'ray_directions')):
         if isinstance(t, torch.Tensor) and t.requires_grad:
             raise NotImplementedError(f'{name} requires grad: the renderer differentiates w.r.t. planes and decoder only')
-    if options.get('output_layout', 'channels_last') != 'channels_last' or int(options.get('depth_clamp_group', 0)) != 0:
-        raise NotImplementedError("autograd supports output_layout='channels_last' and one depth-clamp range per call")
-    if planes.shape[0] != ray_origins.shape[0]:
-        raise NotImplementedError('autograd needs one plane set per camera (no frame batching)')
     _r.pack_decoder(decoder, allow_grad=True)            # validates the decoder's structure before anything is launched
     fc1, fc2 = decoder.net[0], decoder.net[2]
     return _Render.apply(renderer, decoder, options, noise, planes, fc1.weight, fc1.bias, fc2.weight, fc2.bias,

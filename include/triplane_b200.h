@@ -291,18 +291,25 @@ int tpr_sample_3dgrid(const float* grid, int64_t n_grids, int32_t channels, int3
 
 /* ---- backward of a13 (SURVEY.md section 8(f) row 3; the reference gets it from autograd, used by
  *      training/training_loop.py:335,377) ------------------------------------------------------------------------- */
-/* Gradients of L with respect to the tri-planes and the decoder, given g_rgb = dL/d(rgb) [N,M,32] (channels last),
- * g_depth = dL/d(depth) [N,M], g_weight_sum = dL/d(weight_sum) [N,M] of one tpr_render call.
+/* Gradients of L with respect to the tri-planes and the decoder, given g_rgb = dL/d(rgb) [N,M,32] (channels last, whatever
+ * opt->output_layout the forward wrote), g_depth = dL/d(depth) [N,M], g_weight_sum = dL/d(weight_sum) [N,M] of one
+ * tpr_render call.  N = n_img cameras.
  * depths_coarse [N*M,Dc] (tpr_sample_stratified of the forward's jitter) and depths_fine [N*M,Df] (the forward's
  * fine_depths output; NULL when Df = 0) are the sample depths of the forward, constants of the graph exactly as in the
- * reference (VR/renderer.py:198,210: torch.no_grad + detach); depth_range [2] (device) is the forward's depth_range_out
- * (the clamp of VR/ray_marcher.py:50 passes gradient only inside it).  From opt: box_warp, depth_resolution,
- * depth_resolution_importance, white_back, flags (decoder precision of the colour/density recomputation).  One plane set
- * per image (plane_sets = 0) and one clamp range per call only.
+ * reference (VR/renderer.py:198,210: torch.no_grad + detach).  From opt: box_warp, depth_resolution,
+ * depth_resolution_importance, white_back, flags (decoder precision of the colour/density recomputation), and the forward's
+ * frame batching:
+ *   plane_sets = P > 0 (P divides n_img): camera n sampled plane set n % P; planes_packed and g_planes_packed are then
+ *     [P,3,H,W,32] and the gradient of a set is the sum over its cameras.  0: one set per camera (P = N).
+ *   depth_clamp_group = k: 0 = depth_range [2] (device) is the call's (min, max); k > 0 = depth_range holds
+ *     2 * ceil(N / k) floats, the (min, max) of the depths of cameras [j k, j k + k) (the last group may be shorter).  The
+ *     clamp of VR/ray_marcher.py:50 passes gradient only inside the camera's range.  The forward keeps per-group ranges
+ *     in its scratch only; each is the min and max of the group's coarse and importance depths, so a caller reduces those.
  * Either output may be NULL when the caller does not need that gradient (its phase of the kernel is skipped).
- * g_planes_packed [N,3,H,W,32] (the layout of tpr_pack_planes; OVERWRITTEN) and g_decoder_packed
+ * g_planes_packed [P,3,H,W,32] (the layout of tpr_pack_planes; OVERWRITTEN) and g_decoder_packed
  * [tpr_packed_decoder_bytes()] (the layout of tpr_pack_decoder; OVERWRITTEN; convert with tpr_unpack_decoder_grad).
- * scratch: tpr_render_backward_scratch_bytes(n_img, n_rays, Dc + Df) bytes.
+ * scratch: tpr_render_backward_scratch_bytes(n_img, n_rays, Dc + Df) bytes, plus
+ * tpr_backward_deterministic_scratch_bytes(P, height, width) with TPR_BWD_DETERMINISTIC.
  * sample_colours / sample_sigma [N*M,S]: the per-sample decoder outputs kept by tpr_render_train, in ITS layout (both or
  * neither); NULL = re-evaluate them here with the point-query kernel (tpr_run_model), 3 ms more at config 2.
  * sample_features [N*M,S,32]: the summed plane features of every sample, also kept by tpr_render_train; NULL = gather
@@ -350,7 +357,8 @@ int tpr_run_model_backward(const float* planes_packed, int64_t n_img, int32_t he
                            void* scratch, size_t scratch_bytes, void* stream);
 /* Extra scratch of the deterministic backward (TPR_BWD_DETERMINISTIC), on top of tpr_render_backward_scratch_bytes /
  * tpr_run_model_backward_scratch_bytes: the int64 plane-gradient accumulator [N,3,H,W,32] plus 512 per-CTA rows of the
- * packed decoder gradient (a launch in this mode uses at most 512 CTAs) and 256 bytes.  0 for a bad shape. */
+ * packed decoder gradient (a launch in this mode uses at most 512 CTAs) and 256 bytes.  0 for a bad shape.  For
+ * tpr_render_backward with plane_sets = P > 0 pass P as n_img: the accumulator holds one entry per plane set. */
 size_t tpr_backward_deterministic_scratch_bytes(int64_t n_img, int32_t height, int32_t width);
 /* the two stages of tpr_render_backward, stand-alone (tests): the march's backward -- sigma [R,S], colours [R,S,32] of
  * the samples in forward order -> g_sigma [R,S] and the composite weight omega [R,S] of each sample's colour
